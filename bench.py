@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 10 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
     python bench.py --impl reference ...        # the reference's CPU path (oracle restatement) on the host cores
+    python bench.py ... --dump-outputs DIR      # also write what the timed step returned in its last step (see dump_outputs)
 
 Workload (BASELINE.json configs[1], SURVEY 8d): reconstructed run_code/1d_config denoiser (536.8 M params), bf16 compute,
 one step = add_noise -> forward -> MSE -> backward over a synthetic batch of 32 x 752 codec frames with 550 text tokens per
@@ -30,6 +31,7 @@ sys.path.insert(0, ROOT)
 
 CFG = "1d_config"
 BATCH, T_FRAMES = 32, 752
+DUMP_GRAD_SAMPLE = 1 << 23        # gradient elements --dump-outputs writes (32 MB fp32 of the step's 536.8 M)
 FLOP_PER_FRAME = 1.051e9          # fwd+bwd algorithmic FLOPs per codec frame (SURVEY 8d / BASELINE.md section 3)
 METRIC = "denoiser_train_codec_frames_per_sec"
 
@@ -182,8 +184,8 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = min(args.steps, 4)     # ~5 s per step on 8 host threads: keep the arm within a few minutes
-    warm = min(args.warmup, 1)
+    steps = args.steps
+    warm = min(args.warmup, 1)     # ~5 s per step on 8 host threads: one warm-up step is enough on the host
     cb, sec = cpu_reference_step_time(steps, warm)
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": "frames/s", "n_gpus": args.gpus, "steps": steps,
             "warmup": warm, "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -300,6 +302,8 @@ def run_ours(args):
     ms_e2e = timed(e2e_step, args.steps)
     ck = clocks.stop() if rank == 0 else None
     loss_val = float(loss_buf.item())
+    if args.dump_outputs and rank == 0:      # before the full-step leg below moves the weights
+        dump_outputs(args.dump_outputs, model, loss_buf, torch)
     n_buckets = grad_sync.n_buckets_last
 
     # compute-only step at N > 1 (same box, same minute): the step with the gradient exchange switched off -> exposed communication
@@ -663,6 +667,26 @@ def rvq_throughput(dev, torch, ops, hbm_gbs, rank=0, world=1, max_over_ranks=lam
                     "per launch into preallocated buffers", "decode_equals_sequential_codeword_sum": ok}
 
 
+def dump_outputs(out_dir, model, loss, torch):
+    """What the timed step hands its caller after its last step, for comparing two builds output for output (the inputs and
+    weights are seeded, so the same arguments give the same inputs):
+      loss.npy        float32 []    the step's MSE loss
+      grad_sample.npy float32 [N]   DUMP_GRAD_SAMPLE elements of the parameter gradients (param.grad), drawn with a fixed seed from
+                                    all of them flattened and concatenated in named_parameters() order
+      grad_norms.npy  float64 [P]   the L2 norm of every parameter's gradient, same order, so that a change anywhere shows
+    Parameters that receive no gradient (the reference's dead proj_out tensors) are left out of both.  Two runs of the same build
+    agree to rounding, not bit for bit, so compare with a tolerance."""
+    import numpy as np
+    grads = [p.grad for _, p in model.named_parameters() if p.grad is not None]
+    flat = torch.cat([g.reshape(-1) for g in grads])
+    idx = torch.randint(0, flat.numel(), (min(DUMP_GRAD_SAMPLE, flat.numel()),), generator=torch.Generator().manual_seed(0)).sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "grad_sample.npy"), flat[idx.to(flat.device)].cpu().numpy())
+    np.save(os.path.join(out_dir, "grad_norms.npy"), torch.stack([g.double().norm() for g in grads]).cpu().numpy())
+    del flat
+
+
 def gemm_profile(step, model, ops, torch):
     """Duration of the two tensor-core kernel families inside one step, measured live with CUDA events.
     One eager step is run with every pt_gemm / pt_attn_* call recorded (arguments and the tensors behind them are kept alive); the
@@ -761,7 +785,12 @@ def main():
     ap.add_argument("--no-full-step", action="store_true")
     ap.add_argument("--no-rvq", action="store_true")
     ap.add_argument("--no-codec", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed step's outputs of its last step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl ours)")
     protect_stdout()
     if args.impl == "reference":
         run_reference(args)

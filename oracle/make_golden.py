@@ -1,8 +1,9 @@
-"""Generates tests/golden/*.npz by running the UNMODIFIED reference (imported from /root/reference with the diffusers-0.15
-shim of oracle/diffusers_shim first on sys.path) and the transformers restatement of encodec's RVQ.  Run in the build
-container only (the GPU box has no /root/reference):
+"""Generates tests/golden/*.npz by running the UNMODIFIED reference (a checkout of the original project, named by
+$PROMPT_TTS_REFERENCE and imported with the diffusers-0.15 shim of oracle/diffusers_shim first on sys.path) and transformers'
+restatement of encodec (RVQ and SEANet).  The tests read the stored vectors and need neither the reference nor transformers:
 
-    python oracle/make_golden.py            (or `... make_golden.py seanet` for the EnCodec SEANet vectors only)
+    PROMPT_TTS_REFERENCE=<reference checkout> python oracle/make_golden.py
+    python oracle/make_golden.py seanet | transformers        (one set only; transformers needed, the reference not)
 
 TEST INFRASTRUCTURE ONLY.  The vectors pin oracle/ref_model.py and oracle/rvq_oracle.c (tests/test_oracle.py)."""
 import json
@@ -15,13 +16,13 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 sys.path.insert(0, os.path.join(HERE, "diffusers_shim"))
-sys.path.insert(1, "/root/reference")
-sys.path.insert(2, HERE)
-sys.path.insert(3, os.path.join(ROOT, "tests"))
+sys.path.insert(1, HERE)
+sys.path.insert(2, os.path.join(ROOT, "tests"))
 OUT = os.path.join(ROOT, "tests", "golden")
 
 
 def denoiser(cfg_name, B, T, seed):
+    sys.path.insert(1, os.environ["PROMPT_TTS_REFERENCE"])
     import ref_model
     from tts.models import TTSSingleSpeaker          # the reference's own module tree
     from diffusers import DDPMScheduler              # shim: diffusers 0.15 semantics
@@ -105,13 +106,74 @@ def seanet():
     np.savez_compressed(os.path.join(OUT, "seanet_golden.npz"), **out)
 
 
+# (config, samples) of the SEANet stacks tests/test_seanet_host.py pins seanet_oracle on: weights make_weights(cfg, 3), input
+# rng(5).standard_normal((2, 1, samples)) * 0.3
+def seanet_pin_variants():
+    import seanet_oracle as so
+    return ((so.CFG_TINY, 3203), (so.CFG_24KHZ, 3520),
+            (dict(so.CFG_TINY, use_causal_conv=False), 3333),           # the asymmetric padding of ME:159-163 / ME:203-204
+            (dict(so.CFG_TINY, use_conv_shortcut=False), 2900),         # encodec's true_skip
+            (dict(so.CFG_TINY, pad_mode="constant"), 3001),
+            (dict(so.CFG_TINY, num_residual_layers=2, dilation_growth_rate=3), 3200))
+
+
+def seanet_pin_input(S):
+    return (np.random.default_rng(5).standard_normal((2, 1, S)) * 0.3).astype(np.float32)
+
+
+def rvq_full_batch():
+    """One complete reference batch (32 clips x 900 frames, generate_code.py:29-34,94-96): Gaussian codebooks and latents, the
+    tails of the last 12 clips zero-padded."""
+    rs = np.random.RandomState(11)
+    cb = rs.standard_normal((8, 1024, 128)).astype(np.float32)
+    lat = rs.standard_normal((32, 128, 900)).astype(np.float32)
+    lat[20:, :, 650:] = 0.0
+    return cb, lat
+
+
+def transformers_refs():
+    """What transformers computes for the tests that pin the oracles and the RVQ kernels against it:
+    seanet_transformers.npz -- encoder latents and decoder output (decoder fed transformers' latents) of every
+    seanet_pin_variants() stack, with the config each was made with, and the 24 kHz model's encoder / decoder parameter table;
+    rvq_full_batch.npz -- codes of encodec's quantiser on rvq_full_batch() at 6 kbps and the SHA-256 of the bytes of its decode of
+    those codes (the embedding sum is compared bit for bit; 15 MB of it would not fit the repository)."""
+    import hashlib
+    import seanet_oracle as so
+    from transformers import EncodecConfig, EncodecModel
+    from transformers.models.encodec.modeling_encodec import EncodecResidualVectorQuantizer
+    out = {}
+    for i, (cfg, S) in enumerate(seanet_pin_variants()):
+        m = so.to_transformers_model(so.make_weights(cfg, 3), cfg)
+        with torch.no_grad():
+            lat = m.encoder(torch.from_numpy(seanet_pin_input(S))).numpy()
+            wav = m.decoder(torch.from_numpy(lat)).numpy()
+        out.update({f"v{i}_cfg": np.array(json.dumps(cfg)), f"v{i}_S": np.int64(S), f"v{i}_lat": lat, f"v{i}_wav": wav})
+    sd = EncodecModel(EncodecConfig()).state_dict()
+    out["param_shapes_24khz"] = np.array(json.dumps({k: list(v.shape) for k, v in sd.items() if k.startswith(("encoder.", "decoder."))}))
+    np.savez_compressed(os.path.join(OUT, "seanet_transformers.npz"), **out)
+    cb, lat = rvq_full_batch()
+    q = EncodecResidualVectorQuantizer(EncodecConfig())
+    with torch.no_grad():
+        for i in range(8):
+            q.layers[i].codebook.embed.copy_(torch.from_numpy(cb[i]))
+        codes = q.encode(torch.from_numpy(lat), 6.0)                         # [8, B, T]
+        dec = np.ascontiguousarray(q.decode(codes).numpy())                  # [B, 128, T] fp32
+    np.savez_compressed(os.path.join(OUT, "rvq_full_batch.npz"), codes=codes.permute(1, 0, 2).numpy().astype(np.uint16),
+                        dec_sha256=np.array(hashlib.sha256(dec.tobytes()).hexdigest()))
+    print("wrote seanet_transformers, rvq_full_batch")
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
     if sys.argv[1:] == ["seanet"]:
         seanet()
+        sys.exit(0)
+    if sys.argv[1:] == ["transformers"]:
+        transformers_refs()
         sys.exit(0)
     denoiser("tiny", 2, 16, 0)
     denoiser("tiny3", 2, 32, 1)
     rvq("grid", 0, 3, 77, True)
     rvq("gauss", 1, 2, 150, False)
     seanet()
+    transformers_refs()

@@ -195,6 +195,34 @@ def test_reference_arm_prints_one_json_line():
     assert d["e2e"]["value"] == d["value"] and d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: the loss, a gradient sample taken at the same positions every time (in the parameters' logical
+    element order, whatever the layout of the gradient view) and every gradient's norm, as float32 / float64 .npy files within the
+    64 MB a dump may take; --steps below one and a dump of the CPU arm are refused."""
+    import numpy as np
+    import bench
+    assert bench.DUMP_GRAD_SAMPLE * 4 + 4096 * 8 <= 64 << 20
+    monkeypatch.setattr(bench, "DUMP_GRAD_SAMPLE", 16)
+    m = torch.nn.Module()
+    m.a, m.dead, m.b = (torch.nn.Parameter(torch.zeros(s)) for s in ((5, 7), (3,), (11,)))
+    m.a.grad = torch.arange(35.0).reshape(5, 7).t().contiguous().t()      # a non-contiguous view, like a k=3 conv weight's gradient
+    m.b.grad = torch.arange(11.0) + 100
+    values = set(range(35)) | set(range(100, 111))
+    dumps = []
+    for d in (tmp_path / "one", tmp_path / "two"):
+        bench.dump_outputs(str(d), m, torch.tensor(0.25), torch)
+        got = {n: np.load(d / f"{n}.npy") for n in ("loss", "grad_sample", "grad_norms")}
+        assert got["loss"].dtype == np.float32 and got["loss"].shape == () and got["loss"] == 0.25
+        assert got["grad_norms"].dtype == np.float64 and np.allclose(got["grad_norms"], [m.a.grad.norm(), m.b.grad.norm()])
+        s = got["grad_sample"]
+        assert s.dtype == np.float32 and s.shape == (16,) and set(s.tolist()) <= values and (np.diff(s) >= 0).all()
+        dumps.append(s)
+    assert np.array_equal(dumps[0], dumps[1])
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and "error" in r.stderr, (argv, r.stderr[-500:])
+
+
 def test_flop_count_matches_the_survey():
     """tools/count_flops.py walks the module tree of the full config: the roofline denominators of SURVEY 8(d)."""
     sys.path.insert(0, os.path.join(ROOT, "tools"))

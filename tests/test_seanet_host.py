@@ -5,6 +5,7 @@ of libpt_seanet.so, and the kernels' index arithmetic through the host-side grid
 seanet_core.h bodies compiled for the host, so buffer routing, padding and activation placement are checked here without a
 GPU.  The product never constructs it (see test_product_raises_without_gpu)."""
 import ctypes as C
+import json
 import os
 import re
 import subprocess
@@ -19,7 +20,6 @@ sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
 import seanet_oracle as so  # noqa: E402
 from prompt_tts_b200 import codec  # noqa: E402
-from prompt_tts_b200._lib import PtError  # noqa: E402
 
 EMUL_SO = os.path.join(ROOT, "oracle", "_build", "libseanet_emul.so")
 
@@ -64,19 +64,16 @@ def rel(a, b):
 
 # ------------------------------------------------------------------------------------------------ oracle pinning
 def test_oracle_matches_transformers_tiny_and_24khz():
-    import torch
-    variants = ((so.CFG_TINY, 3203), (so.CFG_24KHZ, 3520),
-                (dict(so.CFG_TINY, use_causal_conv=False), 3333),           # the asymmetric padding of ME:159-163 / ME:203-204
-                (dict(so.CFG_TINY, use_conv_shortcut=False), 2900),         # encodec's true_skip
-                (dict(so.CFG_TINY, pad_mode="constant"), 3001),
-                (dict(so.CFG_TINY, num_residual_layers=2, dilation_growth_rate=3), 3200))
-    for cfg, S in variants:
+    """transformers' EncodecModel on the same weights and input, as stored by oracle/make_golden.py (transformers)."""
+    import make_golden as mg
+    g = np.load(os.path.join(ROOT, "tests", "golden", "seanet_transformers.npz"))
+    variants = mg.seanet_pin_variants()
+    assert len(variants) == 6
+    for i, (cfg, S) in enumerate(variants):
+        assert json.loads(str(g[f"v{i}_cfg"])) == json.loads(json.dumps(cfg)) and int(g[f"v{i}_S"]) == S, (i, "regenerate the golden file")
         P = so.make_weights(cfg, 3)
-        m = so.to_transformers_model(P, cfg)
-        x = (np.random.default_rng(5).standard_normal((2, 1, S)) * 0.3).astype(np.float32)
-        with torch.no_grad():
-            lat_ref = m.encoder(torch.from_numpy(x)).numpy()
-            wav_ref = m.decoder(torch.from_numpy(lat_ref)).numpy()
+        x = mg.seanet_pin_input(S)
+        lat_ref, wav_ref = g[f"v{i}_lat"], g[f"v{i}_wav"]
         lat = so.encoder(x, P, cfg)
         assert lat.shape == lat_ref.shape == (2, cfg["hidden_size"], -(-S // 320))
         assert rel(lat, lat_ref) < 1e-5
@@ -86,9 +83,9 @@ def test_oracle_matches_transformers_tiny_and_24khz():
 
 
 def test_oracle_param_table_is_transformers_state_dict():
-    from transformers import EncodecConfig, EncodecModel
-    sd = EncodecModel(EncodecConfig()).state_dict()
-    want = {k: tuple(v.shape) for k, v in sd.items() if k.startswith(("encoder.", "decoder."))}
+    """The encoder / decoder tensors of transformers' EncodecModel(EncodecConfig()), as stored by oracle/make_golden.py."""
+    g = np.load(os.path.join(ROOT, "tests", "golden", "seanet_transformers.npz"))
+    want = {k: tuple(v) for k, v in json.loads(str(g["param_shapes_24khz"])).items()}
     assert so.param_shapes(so.CFG_24KHZ) == want
     # the product's plan names exactly the same tensors
     model_names = []
@@ -198,13 +195,21 @@ def test_argument_validation_needs_no_gpu():
 
 
 def test_product_raises_without_gpu():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    with pytest.raises(PtError):
-        codec.EncodecModel()
-    with pytest.raises(PtError):
-        codec.EncodecModel.encodec_model_24khz(pretrained=False)
+    """Run with no CUDA device visible (CUDA_VISIBLE_DEVICES empty), so that a machine with a GPU checks it too."""
+    code = r'''
+import sys
+sys.path.insert(0, %r)
+import pytest
+from prompt_tts_b200 import codec
+from prompt_tts_b200._lib import PtError
+with pytest.raises(PtError):
+    codec.EncodecModel()
+with pytest.raises(PtError):
+    codec.EncodecModel.encodec_model_24khz(pretrained=False)
+print("OK")
+''' % ROOT
+    r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0 and "OK" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
 
 
 # ------------------------------------------------------------------------------------------------ kernel bodies vs oracle
