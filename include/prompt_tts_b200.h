@@ -29,6 +29,7 @@
  *   pt_codes_affine    codes/1023 -> Normalize(0.5,0.5)            tts/dataloader.py:64,77,168-170
  *   pt_add_noise, pt_mse_*        train-step glue                  train.py:96-98,107
  *   pt_ddpm_step       sampling step (diffusers DDPMScheduler.step; SURVEY 8 row N1, not in the reference tree)
+ *   pt_ddim_step, pt_dpmpp_step   few-step sampling (diffusers DDIMScheduler / DPMSolverMultistepScheduler.step; not in the reference tree)
  */
 #ifndef PROMPT_TTS_B200_H
 #define PROMPT_TTS_B200_H
@@ -227,6 +228,20 @@ int pt_add_noise(const float* x0, const float* noise, const int64_t* t, const fl
  * known != NULL: the first `keep` frames of every length-T row are overwritten from `known` (speech-prompt in-painting). */
 int pt_ddpm_step(const float* eps, const float* xt, const float* noise, const float* known, float* out, int64_t n, int T, int keep,
                  float acp_t, float acp_prev, void* stream);
+/* Few-step sampling, one fused elementwise pass each.  eps, xt, out: n fp32 values in rows of length T (out may alias xt).
+ * Prompt in-painting: frames t < keep of every row are overwritten with p_a * prompt + p_b * prompt_noise, both [n / T, keep]
+ * fp32 (prompt_noise is not read when p_b == 0; p_a = 1, p_b = 0 writes the clean prompt).
+ * pt_ddim_step: diffusers 0.15 DDIMScheduler.step (clip_sample, set_alpha_to_one, raw eps in the direction term); acp_prev = 1 at
+ * the last step; noise is read when eta > 0 (required then).  Fails when eta makes 1 - acp_prev - std^2 negative (eta <= 1 never does).
+ * pt_dpmpp_step: diffusers 0.15 DPMSolverMultistepScheduler.step, "dpmsolver++" with the midpoint second-order update, from
+ * timestep s0 (acp_s0) to t (acp_t); order 2 also uses the previous timestep s1 (acp_s1) and m_prev, the x0 prediction made there.
+ * m_out (optional) receives this step's x0 prediction (x - sigma_s0 eps) / alpha_s0, also in the in-painted frames; it may alias
+ * m_prev. */
+int pt_ddim_step(const float* eps, const float* xt, const float* noise, const float* prompt, const float* prompt_noise, float* out,
+                 int64_t n, int T, int keep, float acp_t, float acp_prev, float eta, float p_a, float p_b, void* stream);
+int pt_dpmpp_step(const float* eps, const float* xt, const float* m_prev, float* m_out, const float* prompt, const float* prompt_noise,
+                  float* out, int64_t n, int T, int keep, float acp_s0, float acp_s1, float acp_t, int order, float p_a, float p_b,
+                  void* stream);
 /* loss += mean((pred - target)^2) ; dpred = 2 (pred - target) / n * gscale ; loss must be zeroed by caller */
 int pt_mse_fwd_bwd(const float* pred, const float* target, float* loss, float* dpred, int64_t n, float gscale, void* stream);
 

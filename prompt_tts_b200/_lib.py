@@ -126,6 +126,8 @@ _SIGS = {
     "add_noise": "ppppppilp",
     "mse_fwd_bwd": "pppplfp",
     "ddpm_step": "pppppliiffp",
+    "ddim_step": "ppppppliifffffp",
+    "dpmpp_step": "pppppppliifffiffp",
     "rvq_encode_ws": "ppppiiiiip",
     "rvq_cb_sq": "ppiiip",
     "rvq_encode_tc": "pppipiiiiip",

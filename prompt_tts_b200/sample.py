@@ -13,11 +13,17 @@ Here the text encoder runs once, the cross-attention K/V projections of its outp
 steps (they do not depend on x or t), one denoiser forward is captured in a CUDA graph and replayed per step, and the
 scheduler step is one fused kernel (`pt_ddpm_step`), optionally in-painting the first `prompt` frames from a noised copy
 of the speech prompt (the builder-defined prompt protocol of SURVEY 8d config 4).
+
+`DDIMSampler` and `DPMSolverSampler` run the same loop with diffusers 0.15's `DDIMScheduler` (default 50 steps) and
+`DPMSolverMultistepScheduler` (DPM-Solver++ order 2, default 20 steps) on the same trained model: one denoiser forward per step,
+so the cost of a sample is proportional to the step count.  Their steps are `pt_ddim_step` / `pt_dpmpp_step`, which in-paint the
+prompt frames inside the kernel.
 """
 from __future__ import annotations
 
-from typing import Dict, Optional
+from typing import Dict, List, Optional
 
+import numpy as np
 import torch
 
 from . import engine as E
@@ -29,13 +35,15 @@ def ddpm_alphas_cumprod(n: int = 1000, beta_start: float = 1e-4, beta_end: float
     return torch.cumprod(1.0 - betas, 0)
 
 
-class DDPMSampler:
-    def __init__(self, model, n_infer: int = 100, n_train: int = 1000, use_graph: bool = True):
+class _Sampler:
+    """The sampling loop every scheduler shares: text encoder once, cross-attention K/V cached, one denoiser forward captured at
+    call 1 and replayed; `_step` is the scheduler's update of x in place from the eps the forward left in `_static["eps"]`."""
+    timesteps: List[int]
+
+    def __init__(self, model, n_infer: int, use_graph: bool):
         self.model = model
-        self.n_infer, self.n_train = n_infer, n_train
-        self.stride = n_train // n_infer
-        self.acp = ddpm_alphas_cumprod(n_train)               # host copy: the step coefficients are scalars per step
-        self.timesteps = [i * self.stride for i in range(n_infer)][::-1]
+        self.n_infer = n_infer
+        self.acp = ddpm_alphas_cumprod()                      # host copy: the step coefficients are scalars per step
         self.use_graph = use_graph
         self.cache = E.get_cache(model)
         self._graph = None
@@ -48,18 +56,26 @@ class DDPMSampler:
         y, _ = self.model.unet._fwd(tape, self._static["x"], self._static["t"], self._enc)
         self._static["eps"].copy_(y)
 
+    def _start(self, x: torch.Tensor, prompt: Optional[torch.Tensor], prompt_noise: Optional[torch.Tensor], keep: int) -> None:
+        """per-call state of the scheduler step"""
+        raise NotImplementedError
+
+    def _step(self, i: int, t: int, x: torch.Tensor, noises: Optional[torch.Tensor], gen: torch.Generator) -> None:
+        raise NotImplementedError
+
     @torch.no_grad()
     def sample(self, ids: torch.Tensor, T: int, x_T: Optional[torch.Tensor] = None, noises: Optional[torch.Tensor] = None,
                prompt: Optional[torch.Tensor] = None, prompt_noise: Optional[torch.Tensor] = None, seed: int = 0,
                return_codes: bool = False, prompt_tokens: Optional[torch.Tensor] = None) -> torch.Tensor:
         """ids int32 [B, Lt]; returns x_0 fp32 [B, C, T] (or int64 codes in [0, 1023] with return_codes).
         x_T / noises[n_infer, B, C, T] / prompt_noise may be given for reproducibility against an oracle; otherwise they are
-        drawn from a generator seeded with `seed`.  prompt fp32 [B, C, P]: clean prompt frames in-painted at every step.
+        drawn from a generator seeded with `seed` (noises is read only at the steps that add noise).  prompt fp32 [B, C, P]:
+        clean prompt frames in-painted at every step, noised to the level the step lands on (clean at the last step).
         prompt_tokens float [B, P, cross_attention_dim] (optional, default off): a speech-prompt encoding appended to the text
         encoding as extra cross-attention tokens -- `Unet1DConditionModel.forward` takes `encoder_hidden_states` of any length
         (unet_1d_condition.py:557); with None the conditioning is exactly the reference's."""
         if not ids.is_cuda:
-            raise ops._lib.PtError("DDPMSampler: inputs must be CUDA tensors; there is no CPU fallback")
+            raise ops._lib.PtError(f"{type(self).__name__}: inputs must be CUDA tensors; there is no CPU fallback")
         dev = ids.device
         B = ids.shape[0]
         Cin = self.model.unet.conv_in.weight.shape[1]
@@ -76,13 +92,12 @@ class DDPMSampler:
         self._static = {"x": x, "t": torch.zeros(B, dtype=torch.int64, device=dev), "eps": torch.empty_like(x)}
         self._graph = None
         keep = 0
-        known = None
         if prompt is not None:
             keep = prompt.shape[-1]
-            known = torch.zeros_like(x)
             if prompt_noise is None:
                 prompt_noise = torch.randn(self.n_infer, B, Cin, keep, device=dev, generator=gen)
-        noise = torch.empty_like(x)
+        self._T = T
+        self._start(x, prompt, prompt_noise, keep)
         for i, t in enumerate(self.timesteps):
             self._static["t"].fill_(t)
             if self.use_graph and i == 1:        # call 0 ran eagerly (fills the K/V cache, warms the weight packs); capture call 1
@@ -95,23 +110,128 @@ class DDPMSampler:
                 self._graph.replay()
             else:
                 self._denoise()
-            t_prev = t - self.stride
-            acp_t = float(self.acp[t])
-            acp_prev = float(self.acp[t_prev]) if t_prev >= 0 else 1.0
-            if t_prev >= 0:
-                if noises is not None:
-                    noise.copy_(noises[i])
-                else:
-                    noise.normal_(generator=gen)
-            if known is not None:
-                # in-paint: the prompt frames of x_{t_prev} are the clean prompt noised to level t_prev (clean at the last step)
-                sa, sb = (acp_prev ** 0.5, (1.0 - acp_prev) ** 0.5) if t_prev >= 0 else (1.0, 0.0)
-                known[..., :keep] = sa * prompt + sb * prompt_noise[i]
-            ops.call("ddpm_step", ops._p(self._static["eps"]), ops._p(x), ops._p(noise if t_prev >= 0 else None), ops._p(known), ops._p(x),
-                     x.numel(), T, keep, acp_t, acp_prev, ops._stream())
+            self._step(i, t, x, noises, gen)
         self._graph = None
         if return_codes:
             codes = torch.empty(x.shape, dtype=torch.int64, device=dev)
             ops.call("codes_affine_inv", ops._p(x), ops._p(codes), x.numel(), ops._stream())
             return codes
         return x
+
+
+class DDPMSampler(_Sampler):
+    def __init__(self, model, n_infer: int = 100, n_train: int = 1000, use_graph: bool = True):
+        super().__init__(model, n_infer, use_graph)
+        self.n_train = n_train
+        self.stride = n_train // n_infer
+        self.acp = ddpm_alphas_cumprod(n_train)
+        self.timesteps = [i * self.stride for i in range(n_infer)][::-1]
+
+    def _start(self, x, prompt, prompt_noise, keep):
+        self._prompt, self._prompt_noise, self._keep = prompt, prompt_noise, keep
+        self._known = torch.zeros_like(x) if prompt is not None else None
+        self._noise = torch.empty_like(x)
+
+    def _step(self, i, t, x, noises, gen):
+        known, noise, keep = self._known, self._noise, self._keep
+        t_prev = t - self.stride
+        acp_t = float(self.acp[t])
+        acp_prev = float(self.acp[t_prev]) if t_prev >= 0 else 1.0
+        if t_prev >= 0:
+            if noises is not None:
+                noise.copy_(noises[i])
+            else:
+                noise.normal_(generator=gen)
+        if known is not None:
+            # in-paint: the prompt frames of x_{t_prev} are the clean prompt noised to level t_prev (clean at the last step)
+            sa, sb = (acp_prev ** 0.5, (1.0 - acp_prev) ** 0.5) if t_prev >= 0 else (1.0, 0.0)
+            known[..., :keep] = sa * self._prompt + sb * self._prompt_noise[i]
+        ops.call("ddpm_step", ops._p(self._static["eps"]), ops._p(x), ops._p(noise if t_prev >= 0 else None), ops._p(known), ops._p(x),
+                 x.numel(), self._T, keep, acp_t, acp_prev, ops._stream())
+
+
+def _check_steps(name: str, n_infer, hi: int) -> int:
+    if isinstance(n_infer, bool) or int(n_infer) != n_infer or not 1 <= int(n_infer) <= hi:
+        raise ValueError(f"{name}: n_infer must be an integer in [1, {hi}], got {n_infer!r}")
+    return int(n_infer)
+
+
+class _KernelPromptSampler(_Sampler):
+    """Samplers whose step kernel in-paints the prompt frames itself, from [B, C, P] and [n_infer, B, C, P] fp32 device buffers."""
+
+    def _start_prompt(self, x, prompt, prompt_noise, keep):
+        self._keep, self._prompt, self._prompt_noise = keep, None, None
+        if prompt is None:
+            return
+        B, C, T = x.shape
+        want = (self.n_infer, B, C, keep)
+        if tuple(prompt.shape) != want[1:] or tuple(prompt_noise.shape) != want or keep > T or not (prompt.is_cuda and prompt_noise.is_cuda):
+            raise ops._lib.PtError(f"{type(self).__name__}: prompt must be a CUDA tensor [B, C, P] = {want[1:]} with P <= T = {T} and "
+                                   f"prompt_noise [n_infer, B, C, P] = {want}; got {tuple(prompt.shape)} / {tuple(prompt_noise.shape)}")
+        self._prompt = prompt.float().contiguous()
+        self._prompt_noise = prompt_noise.float().contiguous()
+
+    def _prompt_args(self, i: int, acp_to: Optional[float]):
+        """pointer / scale arguments of the in-kernel in-painting: the prompt noised to alphas_cumprod `acp_to`, clean for None"""
+        if self._prompt is None:
+            return ops._p(None), ops._p(None), 1.0, 0.0
+        if acp_to is None:
+            return ops._p(self._prompt), ops._p(None), 1.0, 0.0
+        a = torch.tensor(acp_to, dtype=torch.float32)
+        return ops._p(self._prompt), ops._p(self._prompt_noise[i]), float(torch.sqrt(a)), float(torch.sqrt(1 - a))
+
+
+class DDIMSampler(_KernelPromptSampler):
+    """diffusers 0.15 `DDIMScheduler` (clip_sample, set_alpha_to_one, steps_offset 0) over the training schedule: timesteps
+    (n_infer - 1) * r, ..., r, 0 with r = 1000 // n_infer.  eta = 0 is deterministic; eta = 1 adds the DDPM posterior's noise."""
+
+    def __init__(self, model, n_infer: int = 50, eta: float = 0.0, use_graph: bool = True):
+        n_infer = _check_steps("DDIMSampler", n_infer, 1000)
+        if not 0.0 <= eta <= 1.0:
+            raise ValueError(f"DDIMSampler: eta must be in [0, 1] (DDIM's interpolation between deterministic and DDPM noise), got {eta!r}")
+        super().__init__(model, n_infer, use_graph)
+        self.eta = float(eta)
+        self.stride = 1000 // n_infer
+        self.timesteps = [i * self.stride for i in range(n_infer)][::-1]
+
+    def _start(self, x, prompt, prompt_noise, keep):
+        self._start_prompt(x, prompt, prompt_noise, keep)
+        self._noise = torch.empty_like(x) if self.eta > 0 else None
+
+    def _step(self, i, t, x, noises, gen):
+        t_prev = t - self.stride
+        acp_prev = float(self.acp[t_prev]) if t_prev >= 0 else 1.0
+        if self._noise is not None:
+            if noises is not None:
+                self._noise.copy_(noises[i])
+            else:
+                self._noise.normal_(generator=gen)
+        pp, pn, pa, pb = self._prompt_args(i, acp_prev if t_prev >= 0 else None)
+        ops.call("ddim_step", ops._p(self._static["eps"]), ops._p(x), ops._p(self._noise), pp, pn, ops._p(x), x.numel(), x.shape[-1], self._keep,
+                 float(self.acp[t]), acp_prev, self.eta, pa, pb, ops._stream())
+
+
+class DPMSolverSampler(_KernelPromptSampler):
+    """diffusers 0.15 `DPMSolverMultistepScheduler` (DPM-Solver++, order 2, midpoint, lower_order_final): timesteps
+    round(linspace(0, 999, n_infer + 1))[::-1][:-1]; the last step lands at t = 0.  First order at the first step (and at the
+    last one when n_infer < 15), second order from the x0 prediction of the previous step otherwise.  n_infer <= 999: at 1000 the
+    rounded grid repeats a timestep."""
+
+    def __init__(self, model, n_infer: int = 20, use_graph: bool = True):
+        n_infer = _check_steps("DPMSolverSampler", n_infer, 999)
+        super().__init__(model, n_infer, use_graph)
+        self.timesteps = np.linspace(0, 999, n_infer + 1).round()[::-1][:-1].astype(np.int64).tolist()
+
+    def _start(self, x, prompt, prompt_noise, keep):
+        self._start_prompt(x, prompt, prompt_noise, keep)
+        self._m = torch.empty_like(x)            # x0 prediction of the previous step, overwritten with this step's in the kernel
+
+    def _step(self, i, t, x, noises, gen):
+        n = self.n_infer
+        last = i == n - 1
+        t_to = 0 if last else self.timesteps[i + 1]
+        order = 1 if i == 0 or (last and n < 15) else 2
+        acp_s1 = float(self.acp[self.timesteps[i - 1]]) if order == 2 else 0.0
+        pp, pn, pa, pb = self._prompt_args(i, None if last else float(self.acp[t_to]))
+        ops.call("dpmpp_step", ops._p(self._static["eps"]), ops._p(x), ops._p(self._m), ops._p(self._m), pp, pn, ops._p(x), x.numel(),
+                 x.shape[-1], self._keep, float(self.acp[t]), acp_s1, float(self.acp[t_to]), order, pa, pb, ops._stream())

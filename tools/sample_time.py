@@ -1,4 +1,10 @@
-"""Time one DDPMSampler.sample() call at the bench's sampling configuration (B = 64, T = 1504, 100 steps, 225-frame prompt)."""
+"""Time one sample() call at the bench's sampling configuration (B = 64, T = 1504, 225-frame prompt).
+
+    python tools/sample_time.py                          # DDPMSampler, 100 steps
+    python tools/sample_time.py 20 dpm                   # DPMSolverSampler, 20 steps (samplers: ddpm, ddim, dpm)
+    python tools/sample_time.py 100 ddpm 50 ddim 20 dpm --rounds 3    # several configurations, alternating, three rounds
+
+RTF = seconds of GPU time / seconds of audio generated (denoiser only, as bench.py's `sampling` object)."""
 import os
 import sys
 
@@ -7,21 +13,43 @@ import torch  # noqa: E402
 
 import bench  # noqa: E402
 from prompt_tts_b200.models import TTSSingleSpeaker  # noqa: E402
-from prompt_tts_b200.sample import DDPMSampler  # noqa: E402
+from prompt_tts_b200.sample import DDIMSampler, DDPMSampler, DPMSolverSampler  # noqa: E402
 
-steps = int(sys.argv[1]) if len(sys.argv) > 1 else 100
+SAMPLERS = {"ddpm": DDPMSampler, "ddim": DDIMSampler, "dpm": DPMSolverSampler}
+B, T, P = 64, 1504, 225
+
+args = sys.argv[1:]
+rounds = 1
+if "--rounds" in args:
+    k = args.index("--rounds")
+    rounds = int(args[k + 1])
+    del args[k:k + 2]
+runs = []
+while args:
+    steps = int(args.pop(0))
+    kind = args.pop(0) if args and not args[0].isdigit() else "ddpm"
+    if kind not in SAMPLERS:
+        sys.exit(f"unknown sampler {kind!r}: one of {', '.join(SAMPLERS)}")
+    runs.append((kind, steps))
+runs = runs or [("ddpm", 100)]
+
 cfg = bench.load_cfg(bench.CFG)
 dev = torch.device("cuda:0")
 torch.manual_seed(0)
 model = TTSSingleSpeaker(cfg).to(dev).eval()
-inp = bench.synth(cfg, 64, 1504, 4000, dev)
-prompt = inp["x0"][..., :225].contiguous()
-DDPMSampler(model, n_infer=4).sample(inp["ids"], 1504, prompt=prompt, seed=1)
-smp = DDPMSampler(model, n_infer=steps)
-e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-torch.cuda.synchronize()
-e0.record()
-x = smp.sample(inp["ids"], 1504, prompt=prompt, seed=0)
-e1.record()
-torch.cuda.synchronize()
-print(f"sample(): {e0.elapsed_time(e1) / 1e3:.3f} s for {steps} steps, finite {bool(torch.isfinite(x).all())}")
+inp = bench.synth(cfg, B, T, 4000, dev)
+prompt = inp["x0"][..., :P].contiguous()
+DDPMSampler(model, n_infer=4).sample(inp["ids"], T, prompt=prompt, seed=1)      # untimed: first-use costs (allocator pools, weight packs)
+samplers = [(kind, steps, SAMPLERS[kind](model, n_infer=steps)) for kind, steps in runs]
+audio_s = B * T / 75.0
+for r in range(rounds):
+    for kind, steps, smp in samplers:
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        torch.cuda.synchronize()
+        e0.record()
+        x = smp.sample(inp["ids"], T, prompt=prompt, seed=0)
+        e1.record()
+        torch.cuda.synchronize()
+        sec = e0.elapsed_time(e1) / 1e3
+        print(f"{kind} sample(): {sec:.3f} s for {steps} steps ({sec / steps * 1e3:.1f} ms/step), RTF {sec / audio_s:.5f}, "
+              f"finite {bool(torch.isfinite(x).all())}" + (f"  [round {r + 1}]" if rounds > 1 else ""))
