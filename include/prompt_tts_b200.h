@@ -30,6 +30,8 @@
  *   pt_add_noise, pt_mse_*        train-step glue                  train.py:96-98,107
  *   pt_ddpm_step       sampling step (diffusers DDPMScheduler.step; SURVEY 8 row N1, not in the reference tree)
  *   pt_ddim_step, pt_dpmpp_step   few-step sampling (diffusers DDIMScheduler / DPMSolverMultistepScheduler.step; not in the reference tree)
+ *   pt_cond_select_bf16, pt_cfg_combine, pt_rows_add_bias_bf16   classifier-free guidance: condition dropout in training, the
+ *                                 guided eps of diffusers 0.15 pipelines, the null-context cross-attention rows (not in the reference tree)
  */
 #ifndef PROMPT_TTS_B200_H
 #define PROMPT_TTS_B200_H
@@ -242,6 +244,18 @@ int pt_ddim_step(const float* eps, const float* xt, const float* noise, const fl
 int pt_dpmpp_step(const float* eps, const float* xt, const float* m_prev, float* m_out, const float* prompt, const float* prompt_noise,
                   float* out, int64_t n, int T, int keep, float acp_s0, float acp_s1, float acp_t, int order, float p_a, float p_b,
                   void* stream);
+/* Classifier-free guidance (not in the reference tree).  The null condition is an all-zero cross-attention context.
+ * pt_cond_select_bf16: condition dropout, y[b, i] = keep[b] ? x[b, i] : 0 over B rows of per_sample bf16 (a multiple of 8; x and y
+ * 16-byte aligned; y may alias x).  keep: uint8 [B] (torch.bool storage), nonzero keeps the row.  A select, so a NaN / inf in a
+ * dropped row is not propagated.
+ * pt_cfg_combine: eps2 fp32 [2, n] = conditional rows, then unconditional rows; out[i] = u + w * (c - u) rounded step by step
+ * (d = c - u, s = w * d, u + s; no FMA contraction: torch's fp32 result bit for bit).  out may alias eps2.  w must be finite.
+ * pt_rows_add_bias_bf16: y[r, c] = bf16(float(res[r, c]) + bias[c]) over rows x C bf16 (C a multiple of 8; y may alias res): what a
+ * linear layer's fused bias + residual epilogue produces for an all-zero input -- a cross-attention layer's update of rows whose
+ * context is all zero (K = V = 0, so P V = 0 and to_out contributes its bias). */
+int pt_cond_select_bf16(const void* x, const uint8_t* keep, void* y, int B, int64_t per_sample, void* stream);
+int pt_cfg_combine(const float* eps2, float* out, int64_t n, float w, void* stream);
+int pt_rows_add_bias_bf16(const void* res, const float* bias, void* y, int64_t rows, int C, void* stream);
 /* loss += mean((pred - target)^2) ; dpred = 2 (pred - target) / n * gscale ; loss must be zeroed by caller */
 int pt_mse_fwd_bwd(const float* pred, const float* target, float* loss, float* dpred, int64_t n, float gscale, void* stream);
 

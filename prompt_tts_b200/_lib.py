@@ -128,6 +128,9 @@ _SIGS = {
     "ddpm_step": "pppppliiffp",
     "ddim_step": "ppppppliifffffp",
     "dpmpp_step": "pppppppliifffiffp",
+    "cond_select_bf16": "pppilp",
+    "cfg_combine": "pplfp",
+    "rows_add_bias_bf16": "ppplip",
     "rvq_encode_ws": "ppppiiiiip",
     "rvq_cb_sq": "ppiiip",
     "rvq_encode_tc": "pppipiiiiip",

@@ -706,6 +706,38 @@ __global__ void sched_step_kernel(const float* __restrict__ eps, const float* xt
   }
 }
 
+// ------------------------------------------------------------------------------------------------ classifier-free guidance
+// Condition dropout: y[b, :] = keep[b] ? x[b, :] : 0.  A select, not a multiply, so NaN / inf in a dropped row does not survive.
+__global__ void cond_select_bf16_kernel(const bf16* x, const uint8_t* __restrict__ keep, bf16* y, long long nvec, long long vec_per_sample) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += (long long)gridDim.x * blockDim.x) {
+    bf16x8 v = ld16(x + i * 8);
+    if (!keep[i / vec_per_sample]) v.w[0] = v.w[1] = v.w[2] = v.w[3] = 0u;
+    st16(y + i * 8, v);
+  }
+}
+
+// Guided eps (diffusers 0.15 pipelines: uncond + w * (text - uncond)), each operation rounded as torch's fp32 evaluation of that
+// expression rounds it: no FMA contraction.  eps2 = [cond rows | uncond rows]; out may alias the first half.
+__global__ void cfg_combine_kernel(const float* eps2, float* out, long long n, float w) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const float c = eps2[i], u = eps2[n + i];
+    out[i] = __fadd_rn(u, __fmul_rn(w, __fsub_rn(c, u)));
+  }
+}
+
+// What the bf16 GEMM epilogue of `linear(..., bias, residual)` writes for an all-zero accumulator: the staged column term
+// (0 + bias), fmaf(0, alpha, term), + residual, one rounding to bf16 (gemm_tcgen05.cu, non-transposed epilogue).
+__global__ void rows_add_bias_bf16_kernel(const bf16* res, const float* __restrict__ bias, bf16* y, long long nvec, int cvec) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += (long long)gridDim.x * blockDim.x) {
+    const int c0 = (int)(i % cvec) * 8;
+    float f[8];
+    load8(res + i * 8, f);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) f[j] = __fadd_rn(fmaf(0.f, 1.f, __fadd_rn(0.f, __ldg(bias + c0 + j))), f[j]);
+    store8(y + i * 8, f);
+  }
+}
+
 }  // namespace
 
 #define ST ((cudaStream_t)stream)
@@ -941,6 +973,33 @@ extern "C" int pt_dpmpp_step(const float* eps, const float* xt, const float* m_p
   }
   c.p_a = p_a, c.p_b = p_b;
   sched_step_kernel<<<grid_for(n, 256, 4), 256, 0, ST>>>(eps, xt, nullptr, m_prev, m_out, prompt, prompt_noise, out, n, T, keep, c);
+  PT_LAUNCH_CHECK();
+  return PT_OK;
+}
+static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+extern "C" int pt_cond_select_bf16(const void* x, const uint8_t* keep, void* y, int B, int64_t per_sample, void* stream) {
+  PT_REQUIRE(B > 0 && per_sample > 0 && per_sample % 8 == 0, "cond_select_bf16: B=%d per_sample=%lld (per_sample must be a positive multiple of 8)",
+             B, (long long)per_sample);
+  PT_REQUIRE(x != nullptr && y != nullptr && keep != nullptr && aligned16(x) && aligned16(y),
+             "cond_select_bf16: x, y (16-byte aligned) and keep are required");
+  const long long nvec = (long long)B * (per_sample / 8);
+  cond_select_bf16_kernel<<<grid_for(nvec, 256), 256, 0, ST>>>((const bf16*)x, keep, (bf16*)y, nvec, per_sample / 8);
+  PT_LAUNCH_CHECK();
+  return PT_OK;
+}
+extern "C" int pt_cfg_combine(const float* eps2, float* out, int64_t n, float w, void* stream) {
+  PT_REQUIRE(n > 0 && eps2 != nullptr && out != nullptr, "cfg_combine: n=%lld (positive; eps2 and out required)", (long long)n);
+  PT_REQUIRE(isfinite(w), "cfg_combine: guidance scale w=%g must be finite", w);
+  cfg_combine_kernel<<<grid_for(n, 256, 4), 256, 0, ST>>>(eps2, out, n, w);
+  PT_LAUNCH_CHECK();
+  return PT_OK;
+}
+extern "C" int pt_rows_add_bias_bf16(const void* res, const float* bias, void* y, int64_t rows, int C, void* stream) {
+  PT_REQUIRE(rows > 0 && C > 0 && C % 8 == 0, "rows_add_bias_bf16: rows=%lld C=%d (C must be a positive multiple of 8)", (long long)rows, C);
+  PT_REQUIRE(res != nullptr && y != nullptr && bias != nullptr && aligned16(res) && aligned16(y),
+             "rows_add_bias_bf16: res, y (16-byte aligned) and bias are required");
+  const long long nvec = rows * (C / 8);
+  rows_add_bias_bf16_kernel<<<grid_for(nvec, 256), 256, 0, ST>>>((const bf16*)res, bias, (bf16*)y, nvec, C / 8);
   PT_LAUNCH_CHECK();
   return PT_OK;
 }

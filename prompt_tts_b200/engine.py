@@ -140,6 +140,9 @@ class Tape:
         self.kv_cache: Optional[Dict[int, "Var"]] = None
         # cross-attention K/V of all layers as ONE projection of the text encoding: id(attention module) -> (Var, k_off, v_off)
         self.kv_group: Dict[int, Tuple["Var", int, int]] = {}
+        # inference only (classifier-free guidance): rows [0, cond_rows) of the batch are conditioned on the context, the rows after
+        # them have the null (all-zero) context, whose cross-attention update is the to_out bias alone (BasicTransformerBlock._fwd)
+        self.cond_rows: Optional[int] = None
 
     def record(self, fn: Callable[[], None]) -> None:
         if self.recording:
@@ -253,16 +256,21 @@ def _wgrad_gemm(dy2d_op, x2d_op, seg, N: int, K: int, out: torch.Tensor, out_str
 
 # ------------------------------------------------------------------------------------------------ linear / 1x1 conv
 def linear(tape: Tape, x: Var, wparams: Sequence[torch.Tensor], bias: Optional[Sequence[torch.Tensor]] = None,
-           residual: Optional[Var] = None, out_f32: bool = False) -> Var:
+           residual: Optional[Var] = None, out_f32: bool = False, out: Optional[torch.Tensor] = None) -> Var:
     """y[M, N] = x[M, K] @ W^T (+ bias) (+ residual).  `wparams`: one or more fp32 parameters whose rows are stacked
-    (nn.Linear [N, K] or 1x1 nn.Conv1d [N, K, 1])."""
+    (nn.Linear [N, K] or 1x1 nn.Conv1d [N, K, 1]).  out: a contiguous tensor of y's shape and dtype to write into (a row range of
+    a larger activation) instead of a new one."""
     xd = x.data
     K = xd.shape[-1]
     x2 = xd.reshape(-1, K)
     M = x2.shape[0]
     wp = tape.cache.get(wparams, "lin")
     N = wp.shape[0]
-    out = torch.empty(xd.shape[:-1] + (N,), dtype=F32 if out_f32 else BF16, device=xd.device)
+    shape = xd.shape[:-1] + (N,)
+    if out is None:
+        out = torch.empty(shape, dtype=F32 if out_f32 else BF16, device=xd.device)
+    elif out.shape != shape or out.dtype != (F32 if out_f32 else BF16) or not out.is_contiguous():
+        raise ops._lib.PtError(f"linear: out must be a contiguous {tuple(shape)} tensor, got {tuple(out.shape)} {out.dtype}")
     res = residual.data.reshape(M, N) if residual is not None else None
     ops.gemm([ops.operand(x2, True)], [ops.operand(wp, True)], [ops.segment(K)], M, N, out,
              out_mode=OUT_F32 if out_f32 else OUT_BF16, bias=tape.cache.get(bias, "bias") if bias is not None else None, residual=res)
@@ -476,6 +484,38 @@ def attention_core(tape: Tape, q_src: Var, q_off: int, kv_src: Var, k_off: int, 
         accum(q_src, dq_buf, owned=True)
         if not same and not shared_kv:
             accum(kv_src, dkv_buf, owned=True)
+
+    tape.record(bwd)
+    return y
+
+
+# ------------------------------------------------------------------------------------------------ condition dropout
+def cond_keep_mask(keep, B: int, device, who: str) -> torch.Tensor:
+    """Validate a classifier-free-guidance keep mask -- bool / uint8 [B] on the batch's CUDA device, nonzero = keep the text --
+    and return its uint8 view (no copy for a contiguous mask: a captured step reads the caller's buffer at every replay)."""
+    if not torch.is_tensor(keep) or keep.dtype not in (torch.bool, torch.uint8) or tuple(keep.shape) != (B,) \
+            or not keep.is_cuda or keep.device != torch.device(device):
+        desc = f"{keep.dtype} {tuple(keep.shape)} on {keep.device}" if torch.is_tensor(keep) else type(keep).__name__
+        raise ops._lib.PtError(f"{who}: cond_keep must be a bool or uint8 tensor [B] = [{B}] on {device}, got {desc}")
+    keep = keep.contiguous()
+    return keep.view(torch.uint8) if keep.dtype == torch.bool else keep
+
+
+def cond_select(tape: Tape, enc: Var, keep: torch.Tensor) -> Var:
+    """Condition dropout on a text encoding [B, L, D]: rows b with keep[b] == 0 become the null (all-zero) context.  The backward
+    applies the same selection to the gradient, so a dropped sample sends nothing back to the text encoder."""
+    ed = enc.data
+    B = ed.shape[0]
+    per = ed[0].numel()
+    y = Var(torch.empty_like(ed))
+    ops.call("cond_select_bf16", ops._p(ed), ops._p(keep), ops._p(y.data), B, per, ops._stream())
+
+    def bwd():
+        if y.grad is None:
+            return
+        g = y.grad if y.owned else torch.empty_like(y.grad)
+        ops.call("cond_select_bf16", ops._p(y.grad), ops._p(keep), ops._p(g), B, per, ops._stream())
+        accum(enc, g, owned=True)
 
     tape.record(bwd)
     return y

@@ -8,9 +8,11 @@ arithmetic goes through `prompt_tts_b200.engine` (hand-written sm_100a kernels).
 """
 from __future__ import annotations
 
+import torch
 from torch import nn
 
 from .. import engine as E
+from .. import ops
 
 
 class Attention(nn.Module):
@@ -29,8 +31,9 @@ class Attention(nn.Module):
         self.to_v = nn.Linear(ctx, inner, bias=False)
         self.to_out = nn.ModuleList([nn.Linear(inner, query_dim), nn.Dropout(dropout)])
 
-    def _fwd(self, tape, hn: E.Var, ctx, residual: E.Var) -> E.Var:
-        """hn: normed hidden states [B, L, C]; ctx: encoder states Var [B, Lk, Cctx] or None (self-attention)."""
+    def _fwd(self, tape, hn: E.Var, ctx, residual: E.Var, out=None) -> E.Var:
+        """hn: normed hidden states [B, L, C]; ctx: encoder states Var [B, Lk, Cctx] or None (self-attention).
+        out: optional destination of the result (E.linear)."""
         C = self.inner
         if ctx is None:
             qkv = E.linear(tape, hn, [self.to_q.weight, self.to_k.weight, self.to_v.weight])      # fused QKV GEMM
@@ -48,7 +51,7 @@ class Attention(nn.Module):
                 if tape.kv_cache is not None and not tape.recording:
                     tape.kv_cache[id(self)] = kv
             o = E.attention_core(tape, q, 0, kv, 0, C, self.heads, C)
-        return E.linear(tape, o, [self.to_out[0].weight], [self.to_out[0].bias], residual=residual)
+        return E.linear(tape, o, [self.to_out[0].weight], [self.to_out[0].bias], residual=residual, out=out)
 
 
 class GEGLU(nn.Module):
@@ -94,10 +97,32 @@ class BasicTransformerBlock(nn.Module):
         n = E.layernorm(tape, h, self.norm1.weight, self.norm1.bias)
         h = self.attn1._fwd(tape, n, None, h)
         if self.attn2 is not None:
-            n = E.layernorm(tape, h, self.norm2.weight, self.norm2.bias)
-            h = self.attn2._fwd(tape, n, enc, h)
+            if tape.cond_rows is not None:
+                h = self._cross_guided(tape, h, enc)
+            else:
+                n = E.layernorm(tape, h, self.norm2.weight, self.norm2.bias)
+                h = self.attn2._fwd(tape, n, enc, h)
         n = E.layernorm(tape, h, self.norm3.weight, self.norm3.bias)
         return self.ff._fwd(tape, n, h)
+
+    def _cross_guided(self, tape, h: E.Var, enc) -> E.Var:
+        """h += attn2(LN2 h, ctx) for a classifier-free-guidance batch (inference only): rows [0, Bc) of h (Bc = tape.cond_rows)
+        attend to `enc` [Bc, Lk, Cctx]; the rows after them have the null context, an all-zero one.  For those, K = V = 0 (to_k and
+        to_v have no bias), the softmax weights are uniform and P V = 0, so to_out's GEMM sees a zero operand and its epilogue
+        writes bf16(h + bias): that is computed directly (pt_rows_add_bias_bf16), with no K / V, attention or GEMM for those rows.
+        LN2, to_q, the attention and to_out run on the conditional row prefix only, to_out writing into the prefix of the output."""
+        assert not tape.recording, "the null-context shortcut of guided sampling is inference-only"
+        Bc = tape.cond_rows
+        hd = h.data
+        Bt, L, C = hd.shape
+        assert 0 < Bc < Bt and enc.data.shape[0] == Bc, (Bc, Bt, tuple(enc.data.shape))
+        out = torch.empty_like(hd)
+        hc = E.Var(hd[:Bc], needs_grad=False)
+        n = E.layernorm(tape, hc, self.norm2.weight, self.norm2.bias)
+        self.attn2._fwd(tape, n, enc, hc, out=out[:Bc])
+        ops.call("rows_add_bias_bf16", ops._p(hd[Bc:]), ops._p(self.attn2.to_out[0].bias.detach()), ops._p(out[Bc:]),
+                 (Bt - Bc) * L, C, ops._stream())
+        return E.Var(out)
 
 
 class Timesteps(nn.Module):

@@ -115,15 +115,21 @@ class TTSSingleSpeaker(nn.Module):
                                          up_block_types=config["up_block_types"], cross_attention_dim=config["cross_attention_dim"])
 
     def forward(self, sample: torch.FloatTensor, timestep: Union[torch.Tensor, float, int], text_seq_ids: torch.Tensor,
-                attention_mask: torch.Tensor, cross_attention_kwargs: Optional[Dict[str, Any]] = None, return_dict: bool = True):
+                attention_mask: torch.Tensor, cross_attention_kwargs: Optional[Dict[str, Any]] = None, return_dict: bool = True,
+                *, cond_keep: Optional[torch.Tensor] = None):
+        """cond_keep (not in the reference): optional bool / uint8 [B] CUDA mask for classifier-free guidance training; samples
+        where it is 0 see the null condition (an all-zero text encoding) and send no gradient to the text encoder."""
         if not sample.is_cuda:
             raise ops._lib.PtError("TTSSingleSpeaker: inputs must be CUDA tensors; there is no CPU fallback")
         t = Unet1DConditionModel._timesteps(timestep, sample.shape[0], sample.device)
+        keep = E.cond_keep_mask(cond_keep, sample.shape[0], sample.device, "TTSSingleSpeaker") if cond_keep is not None else None
         ids = text_seq_ids.to(device=sample.device, dtype=torch.int32).contiguous()
         params = [p for p in self.parameters()]
 
         def runner(tape, s):
             enc = self.text_encoder._fwd(tape, ids)
+            if keep is not None:
+                enc = E.cond_select(tape, enc, keep)
             y, seed = self.unet._fwd(tape, s.detach().float().contiguous(), t, enc)
             return (y,), seed, lambda: [None]
 

@@ -18,9 +18,17 @@ of the speech prompt (the builder-defined prompt protocol of SURVEY 8d config 4)
 `DPMSolverMultistepScheduler` (DPM-Solver++ order 2, default 20 steps) on the same trained model: one denoiser forward per step,
 so the cost of a sample is proportional to the step count.  Their steps are `pt_ddim_step` / `pt_dpmpp_step`, which in-paint the
 prompt frames inside the kernel.
+
+Classifier-free guidance (`sample(..., guidance_scale=w)`, all three samplers) follows diffusers 0.15's pipelines: with w > 1 each
+step runs the denoiser once at batch 2B -- rows [0, B) conditioned on the text, rows [B, 2B) on the null condition (an all-zero
+context, what condition dropout trains: `DenoiserTrainStep(..., cond_keep=)`) -- and the step uses
+eps = eps_u + w (eps_c - eps_u) (`pt_cfg_combine`).  The null rows' cross-attention is exactly to_out's bias added to the residual
+(ldm/attention.py:BasicTransformerBlock._cross_guided), so it is computed as that.  w = 1 (the default) is the unguided loop.
 """
 from __future__ import annotations
 
+import math
+import numbers
 from typing import Dict, List, Optional
 
 import numpy as np
@@ -33,6 +41,12 @@ from . import ops
 def ddpm_alphas_cumprod(n: int = 1000, beta_start: float = 1e-4, beta_end: float = 0.02) -> torch.Tensor:
     betas = torch.linspace(beta_start, beta_end, n, dtype=torch.float32)
     return torch.cumprod(1.0 - betas, 0)
+
+
+def _check_guidance(name: str, w) -> float:
+    if isinstance(w, bool) or not isinstance(w, numbers.Real) or not math.isfinite(float(w)) or float(w) < 1.0:
+        raise ValueError(f"{name}: guidance_scale must be a finite real number >= 1 (1 = no guidance), got {w!r}")
+    return float(w)
 
 
 class _Sampler:
@@ -49,12 +63,22 @@ class _Sampler:
         self._graph = None
         self._static: Dict[str, torch.Tensor] = {}
 
-    # ---- one denoiser forward on static buffers (x, t) -> eps, with the text encoding and its K/V projections held fixed
+    # ---- one denoiser forward on static buffers (x, t) -> eps, with the text encoding and its K/V projections held fixed.
+    # Guided: x2 = [x | copy of x] at batch 2B, the second half with the null condition, eps = the guided combination of the halves.
     def _denoise(self) -> None:
         tape = E.Tape(self.cache, recording=False)
         tape.kv_cache = self._kv
-        y, _ = self.model.unet._fwd(tape, self._static["x"], self._static["t"], self._enc)
-        self._static["eps"].copy_(y)
+        x2 = self._static.get("x2")
+        if x2 is None:
+            y, _ = self.model.unet._fwd(tape, self._static["x"], self._static["t"], self._enc)
+            self._static["eps"].copy_(y)
+            return
+        B = x2.shape[0] // 2
+        x2[B:].copy_(x2[:B])
+        tape.cond_rows = B
+        y, _ = self.model.unet._fwd(tape, x2, self._static["t"], self._enc)
+        eps = self._static["eps"]
+        ops.call("cfg_combine", ops._p(y), ops._p(eps), eps.numel(), self._w, ops._stream())
 
     def _start(self, x: torch.Tensor, prompt: Optional[torch.Tensor], prompt_noise: Optional[torch.Tensor], keep: int) -> None:
         """per-call state of the scheduler step"""
@@ -66,14 +90,17 @@ class _Sampler:
     @torch.no_grad()
     def sample(self, ids: torch.Tensor, T: int, x_T: Optional[torch.Tensor] = None, noises: Optional[torch.Tensor] = None,
                prompt: Optional[torch.Tensor] = None, prompt_noise: Optional[torch.Tensor] = None, seed: int = 0,
-               return_codes: bool = False, prompt_tokens: Optional[torch.Tensor] = None) -> torch.Tensor:
+               return_codes: bool = False, prompt_tokens: Optional[torch.Tensor] = None, guidance_scale: float = 1.0) -> torch.Tensor:
         """ids int32 [B, Lt]; returns x_0 fp32 [B, C, T] (or int64 codes in [0, 1023] with return_codes).
         x_T / noises[n_infer, B, C, T] / prompt_noise may be given for reproducibility against an oracle; otherwise they are
         drawn from a generator seeded with `seed` (noises is read only at the steps that add noise).  prompt fp32 [B, C, P]:
         clean prompt frames in-painted at every step, noised to the level the step lands on (clean at the last step).
         prompt_tokens float [B, P, cross_attention_dim] (optional, default off): a speech-prompt encoding appended to the text
         encoding as extra cross-attention tokens -- `Unet1DConditionModel.forward` takes `encoder_hidden_states` of any length
-        (unet_1d_condition.py:557); with None the conditioning is exactly the reference's."""
+        (unet_1d_condition.py:557); with None the conditioning is exactly the reference's.
+        guidance_scale w >= 1: classifier-free guidance for w > 1 (module docstring); x_T, noises, the prompt and prompt tokens act
+        on the B guided rows exactly as without guidance.  The model should have been trained with condition dropout."""
+        w = _check_guidance(type(self).__name__, guidance_scale)
         if not ids.is_cuda:
             raise ops._lib.PtError(f"{type(self).__name__}: inputs must be CUDA tensors; there is no CPU fallback")
         dev = ids.device
@@ -81,6 +108,13 @@ class _Sampler:
         Cin = self.model.unet.conv_in.weight.shape[1]
         gen = torch.Generator(device=dev).manual_seed(seed)
         x = x_T.clone().float() if x_T is not None else torch.randn(B, Cin, T, device=dev, generator=gen)
+        guided = w > 1.0
+        x2 = None
+        if guided:      # the sampler's x is the first half of the 2B-row denoiser input: the step kernels update it in place
+            x2 = torch.empty(2 * B, Cin, T, device=dev)
+            x2[:B].copy_(x)
+            x = x2[:B]
+        self._w = w
         # text encoder once; K/V of every cross-attention layer are filled in by the first denoiser call and then reused
         tape = E.Tape(self.cache, recording=False)
         self._enc = self.model.text_encoder._fwd(tape, ids.to(torch.int32).contiguous())
@@ -89,7 +123,9 @@ class _Sampler:
                 raise ops._lib.PtError(f"prompt_tokens must be [B, P, {self._enc.data.shape[2]}], got {tuple(prompt_tokens.shape)}")
             self._enc = E.Var(torch.cat([self._enc.data, ops.cast_bf16(prompt_tokens.float().contiguous())], dim=1), needs_grad=False)
         self._kv: Dict[int, E.Var] = {}
-        self._static = {"x": x, "t": torch.zeros(B, dtype=torch.int64, device=dev), "eps": torch.empty_like(x)}
+        self._static = {"x": x, "t": torch.zeros(2 * B if guided else B, dtype=torch.int64, device=dev), "eps": torch.empty_like(x)}
+        if guided:
+            self._static["x2"] = x2
         self._graph = None
         keep = 0
         if prompt is not None:
@@ -116,7 +152,7 @@ class _Sampler:
             codes = torch.empty(x.shape, dtype=torch.int64, device=dev)
             ops.call("codes_affine_inv", ops._p(x), ops._p(codes), x.numel(), ops._stream())
             return codes
-        return x
+        return x.clone() if guided else x      # guided: not a view that keeps the 2B-row buffer alive
 
 
 class DDPMSampler(_Sampler):

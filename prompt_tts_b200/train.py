@@ -8,6 +8,10 @@
 whole step can be captured in one CUDA graph; parameter gradients land in `param.grad` (fp32 views of one flat buffer with
 the reference's logical shapes), so the reference's `clip_grad_norm_` / `AdamW` lines keep working on top of it.  As with
 `zero_grad()` after every optimiser step in the reference (train.py:120), each accumulation window starts from zero.
+
+Classifier-free guidance training (not in the reference tree): `cond_keep` (bool [B]) replaces the text encoding of the samples
+where it is False with the null condition, an all-zero context, before the denoiser sees it (condition dropout).  The caller draws
+the mask each step, e.g. `torch.rand(B, device=dev) >= p_uncond`, as it draws `noise` and `t`.
 """
 from __future__ import annotations
 
@@ -68,10 +72,14 @@ class DenoiserTrainStep:
             ids = ids.to(torch.int32).contiguous()
         return x0, noise, t, ids
 
-    def __call__(self, x0, noise, t, ids, mask=None, loss_out: Optional[torch.Tensor] = None, gscale: float = 1.0):
+    def __call__(self, x0, noise, t, ids, mask=None, loss_out: Optional[torch.Tensor] = None, gscale: float = 1.0,
+                 cond_keep: Optional[torch.Tensor] = None):
         """x0, noise fp32 [B, C, T]; t int64 [B] in [0, 1000); ids int32 [B, Lt] (other integer / float dtypes are converted).
+        cond_keep: optional bool / uint8 [B] on the same device, 0 = train this sample unconditionally (all-zero text context);
+        read from device memory, so a captured step replays with whatever mask was last written into the same buffer.
         Returns the loss of this micro-batch (0-d fp32 CUDA tensor)."""
         x0, noise, t, ids = self._check(x0, noise, t, ids)
+        keep = E.cond_keep_mask(cond_keep, x0.shape[0], x0.device, "DenoiserTrainStep") if cond_keep is not None else None
         if self.sa is None:
             self.sa, self.sb = ddpm_tables(device=x0.device)
         first = self.micro == 0
@@ -84,6 +92,8 @@ class DenoiserTrainStep:
         tape = E.Tape(self.cache, recording=True)
         self.grad_sync.attach(tape, zero=first, sync=last)
         enc = self.model.text_encoder._fwd(tape, ids)
+        if keep is not None:
+            enc = E.cond_select(tape, enc, keep)
         pred, seed = self.model.unet._fwd(tape, xt, t, enc)
         loss = torch.zeros((), dtype=torch.float32, device=x0.device) if loss_out is None else loss_out.zero_()
         dpred = torch.empty_like(pred)

@@ -24,9 +24,14 @@ def lin_flops(m: nn.Linear, rows: int) -> float:
     return 2.0 * rows * m.weight.shape[0] * m.weight.shape[1]
 
 
-def block_flops(blk, L: int, Lctx: int) -> float:
-    """BasicTransformerBlock on L tokens with a context of Lctx tokens."""
+def block_flops(blk, L: int, Lctx: int, parts=None) -> float:
+    """BasicTransformerBlock on L tokens with a context of Lctx tokens.  parts (optional dict): accumulates the cross-attention's
+    work on the hidden states ("cross_x": to_q, attention, to_out) and on the context ("cross_kv": to_k, to_v)."""
     f = 0.0
+    if parts is not None and blk.attn2 is not None:
+        a = blk.attn2
+        parts["cross_x"] = parts.get("cross_x", 0.0) + lin_flops(a.to_q, L) + lin_flops(a.to_out[0], L) + 4.0 * L * Lctx * a.inner
+        parts["cross_kv"] = parts.get("cross_kv", 0.0) + lin_flops(a.to_k, Lctx) + lin_flops(a.to_v, Lctx)
     for attn, lk, rows_kv in ((blk.attn1, L, L), (blk.attn2, Lctx, Lctx)):
         if attn is None:
             continue
@@ -43,12 +48,12 @@ def resnet_flops(r, L: int) -> float:
     return f
 
 
-def transformer1d_flops(t: Transformer1DModel, L: int, Lctx: int) -> float:
-    return conv_flops(t.proj_in, L) + sum(block_flops(b, L, Lctx) for b in t.transformer_blocks)   # proj_out never runs
+def transformer1d_flops(t: Transformer1DModel, L: int, Lctx: int, parts=None) -> float:
+    return conv_flops(t.proj_in, L) + sum(block_flops(b, L, Lctx, parts) for b in t.transformer_blocks)   # proj_out never runs
 
 
-def forward_flops(model: TTSSingleSpeaker, T: int, Lt: int):
-    """Forward FLOPs per sample: (text encoder, UNet)."""
+def forward_flops(model: TTSSingleSpeaker, T: int, Lt: int, parts=None):
+    """Forward FLOPs per sample: (text encoder, UNet).  parts: see block_flops (UNet cross-attention only)."""
     text = sum(block_flops(b, Lt, Lt) for b in model.text_encoder.transformer_blocks)
     u = model.unet
     L = T
@@ -58,20 +63,20 @@ def forward_flops(model: TTSSingleSpeaker, T: int, Lt: int):
         for i, r in enumerate(blk.resnets):
             f += resnet_flops(r, L)
             if attns is not None:
-                f += transformer1d_flops(attns[i], L, Lt)
+                f += transformer1d_flops(attns[i], L, Lt, parts)
         if getattr(blk, "downsamplers", None) is not None:
             L = (L - 1) // 2 + 1
             f += sum(conv_flops(d.conv, L) for d in blk.downsamplers)
     if u.mid_block is not None:
         f += resnet_flops(u.mid_block.resnets[0], L)
         for a, r in zip(u.mid_block.attentions, u.mid_block.resnets[1:]):
-            f += transformer1d_flops(a, L, Lt) + resnet_flops(r, L)
+            f += transformer1d_flops(a, L, Lt, parts) + resnet_flops(r, L)
     for blk in u.up_blocks:
         attns = getattr(blk, "attentions", None)
         for i, r in enumerate(blk.resnets):
             f += resnet_flops(r, L)
             if attns is not None:
-                f += transformer1d_flops(attns[i], L, Lt)
+                f += transformer1d_flops(attns[i], L, Lt, parts)
         if getattr(blk, "upsamplers", None) is not None:
             L *= 2
             f += sum(conv_flops(up.conv, L) for up in blk.upsamplers)
@@ -92,6 +97,12 @@ def main():
     print(f"forward + backward (3x): {3 * fwd / 1e9:.1f} GFLOP / sample = {3 * fwd / T / 1e9:.3f} GFLOP / frame")
     print(f"train step, batch {B}: {3 * fwd * B / 1e12:.2f} TFLOP;  at 1391 TFLOP/s sustained: {3 * fwd * B / 1391e12 * 1e3:.1f} ms")
     print(f"sampling, 100 steps: {(text + 100 * unet) / 1e12:.2f} TFLOP / utterance")
+    parts = {}
+    forward_flops(model, T, Lt, parts)
+    step = unet - parts["cross_kv"]       # a sampling step: the context's K / V are projected once per sample() call
+    guided = 2 * step - parts["cross_x"]  # classifier-free guidance: the null-context rows skip to_q, attention and to_out
+    print(f"sampling step per sample: {step / 1e9:.1f} GFLOP (cross-attention on x: {parts['cross_x'] / 1e9:.1f}); guided "
+          f"(2 rows, null-context cross-attention skipped): {guided / 1e9:.1f} GFLOP = {guided / step:.3f} x unguided")
 
 
 if __name__ == "__main__":
