@@ -32,6 +32,8 @@
  *   pt_ddim_step, pt_dpmpp_step   few-step sampling (diffusers DDIMScheduler / DPMSolverMultistepScheduler.step; not in the reference tree)
  *   pt_cond_select_bf16, pt_cfg_combine, pt_rows_add_bias_bf16   classifier-free guidance: condition dropout in training, the
  *                                 guided eps of diffusers 0.15 pipelines, the null-context cross-attention rows (not in the reference tree)
+ *   pt_ema_prepare, pt_adamw_ema_step_dev, pt_ema_swap   EMA of the weights (diffusers 0.15 training_utils.EMAModel; not in the
+ *                                 reference tree)
  */
 #ifndef PROMPT_TTS_B200_H
 #define PROMPT_TTS_B200_H
@@ -313,6 +315,28 @@ int pt_sumsq_partials(const void* x, int x_is_bf16, int64_t n, float* partials, 
 int pt_adamw_prepare_det(float* state, const float* partials, int nparts, void* stream);
 int pt_adamw_step_dev(float* p, const void* g, int g_is_bf16, float* m, float* v, void* w_bf16, int64_t n, const float* state,
                       void* stream);
+
+/* Exponential moving average of the weights (diffusers 0.15 training_utils.EMAModel; not in the reference tree).
+ * `ema_state` = PT_EMA_STATE_DOUBLES fp64 words.  The host writes the hyper-parameter slots (PT_EMA_DECAY .. PT_EMA_POWER;
+ * PT_EMA_USE_WARMUP is 0 or 1) and zeroes PT_EMA_STEP.  pt_ema_prepare (one thread) increments the optimisation step (an integer
+ * held in a double) and evaluates, in double precision and in diffusers' order,
+ *   step = max(0, optimization_step - update_after_step - 1)
+ *   decay = step <= 0 ? 0 : use_warmup ? 1 - (1 + step / inv_gamma) ^ -power : (1 + step) / (10 + step)
+ *   decay = max(min(decay, decay_max), min_decay)
+ * and leaves decay in PT_EMA_CUR_DECAY and float(1 - decay) in PT_EMA_COEF.  Nothing host-side is baked into a launch, so a captured
+ * step replays as the next EMA step.
+ * pt_adamw_ema_step_dev: pt_adamw_step_dev, and then, with the updated p, ema = ema - c * (ema - p), c = PT_EMA_COEF, rounded step by
+ * step (no FMA contraction: torch's fp32 `ema.sub_(c * (ema - p))` bit for bit).
+ * pt_ema_swap: exchanges p and ema element by element and writes bf16(new p) into w_bf16 (required), in one pass.
+ * n: a positive multiple of 4 for the last two. */
+enum {
+  PT_EMA_DECAY = 0, PT_EMA_MIN_DECAY, PT_EMA_UPDATE_AFTER, PT_EMA_USE_WARMUP, PT_EMA_INV_GAMMA, PT_EMA_POWER, PT_EMA_STEP,
+  PT_EMA_CUR_DECAY, PT_EMA_COEF, PT_EMA_STATE_DOUBLES = 16
+};
+int pt_ema_prepare(double* ema_state, void* stream);
+int pt_adamw_ema_step_dev(float* p, const void* g, int g_is_bf16, float* m, float* v, void* w_bf16, float* ema, int64_t n,
+                          const float* state, const double* ema_state, void* stream);
+int pt_ema_swap(float* p, float* ema, void* w_bf16, int64_t n, void* stream);
 
 #ifdef __cplusplus
 }

@@ -146,6 +146,9 @@ _SIGS = {
     "sumsq_partials": "pilpip",
     "adamw_prepare_det": "ppip",
     "adamw_step_dev": "ppippplpp",
+    "ema_prepare": "pp",
+    "adamw_ema_step_dev": "ppipppplppp",
+    "ema_swap": "ppplp",
 }
 _CT = {"p": C.c_void_p, "i": C.c_int, "l": C.c_int64, "f": C.c_float}
 EXPORTS = ["pt_version", "pt_last_error", "pt_launch_count", "pt_gemm_last_tile", "pt_rvq_encode_tc_scratch_bytes"] + ["pt_" + k for k in _SIGS]

@@ -600,16 +600,22 @@ __global__ void adamw_prepare_kernel(float* __restrict__ st, const float* __rest
 
 // p, g, m, v fp32 flat buffers in one common layout; w (optional) the bf16 shadow of p in the same layout: the GEMM operands are
 // views of it, so the updated weights need no re-pack pass.  4 elements per thread per iteration (n % 4 == 0).
-template <bool G_BF16>
+// EMA: e (same layout) = e - c * (e - p_new) with c = float(1 - decay) from pt_ema_prepare; the update costs 8 bytes per element
+// here against 12 in a pass of its own.  The EMA arguments come last so that the two plain instantiations keep their code.
+template <bool G_BF16, bool EMA>
 __global__ void __launch_bounds__(256) adamw_dev_kernel(float* __restrict__ p, const void* __restrict__ gv, float* __restrict__ m,
                                                         float* __restrict__ v, bf16* __restrict__ w, long long n4,
-                                                        const float* __restrict__ st) {
+                                                        const float* __restrict__ st, float* __restrict__ e,
+                                                        const double* __restrict__ est) {
   const float clip = st[PT_OPT_CLIP], step_size = st[PT_OPT_STEP_SIZE], isb2 = st[PT_OPT_INV_SQRT_BC2], decay = st[PT_OPT_DECAY];
   const float b1 = st[PT_OPT_BETA1], b2 = st[PT_OPT_BETA2], eps = st[PT_OPT_EPS];
+  const float c = EMA ? (float)est[PT_EMA_COEF] : 0.f;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
     float4 pi = reinterpret_cast<const float4*>(p)[i];
     float4 mi = reinterpret_cast<const float4*>(m)[i];
     float4 vi = reinterpret_cast<const float4*>(v)[i];
+    float4 ei;
+    if (EMA) ei = reinterpret_cast<const float4*>(e)[i];
     float gi[4];
     if (G_BF16) {
       const uint2 t = reinterpret_cast<const uint2*>(gv)[i];
@@ -633,6 +639,36 @@ __global__ void __launch_bounds__(256) adamw_dev_kernel(float* __restrict__ p, c
     reinterpret_cast<float4*>(m)[i] = make_float4(mm[0], mm[1], mm[2], mm[3]);
     reinterpret_cast<float4*>(v)[i] = make_float4(vv[0], vv[1], vv[2], vv[3]);
     if (w != nullptr) reinterpret_cast<uint2*>(w)[i] = make_uint2(f2_to_bf2(pp[0], pp[1]), f2_to_bf2(pp[2], pp[3]));
+    if (EMA) {      // diffusers: s_param.sub_(one_minus_decay * (s_param - param)), three fp32 roundings
+      float ee[4] = {ei.x, ei.y, ei.z, ei.w};
+#pragma unroll
+      for (int j = 0; j < 4; ++j) ee[j] = __fsub_rn(ee[j], __fmul_rn(c, __fsub_rn(ee[j], pp[j])));
+      reinterpret_cast<float4*>(e)[i] = make_float4(ee[0], ee[1], ee[2], ee[3]);
+    }
+  }
+}
+
+// diffusers 0.15 EMAModel.step's bookkeeping and get_decay, in its order and in double precision (python floats)
+__global__ void ema_prepare_kernel(double* __restrict__ st) {
+  const double opt_step = st[PT_EMA_STEP] + 1.0;
+  st[PT_EMA_STEP] = opt_step;
+  const double step = fmax(0.0, opt_step - st[PT_EMA_UPDATE_AFTER] - 1.0);
+  double decay = 0.0;
+  if (step > 0.0) {
+    decay = st[PT_EMA_USE_WARMUP] != 0.0 ? 1.0 - pow(1.0 + step / st[PT_EMA_INV_GAMMA], -st[PT_EMA_POWER]) : (1.0 + step) / (10.0 + step);
+    decay = fmax(fmin(decay, st[PT_EMA_DECAY]), st[PT_EMA_MIN_DECAY]);
+  }
+  st[PT_EMA_CUR_DECAY] = decay;
+  st[PT_EMA_COEF] = (double)(float)(1.0 - decay);
+}
+
+// master <-> EMA exchange; the GEMM operands (w = bf16 shadow of p) follow the new p
+__global__ void ema_swap_kernel(float4* __restrict__ p, float4* __restrict__ e, uint2* __restrict__ w, long long n4) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
+    const float4 a = p[i], b = e[i];
+    p[i] = b;
+    e[i] = a;
+    w[i] = make_uint2(f2_to_bf2(b.x, b.y), f2_to_bf2(b.z, b.w));
   }
 }
 
@@ -1054,9 +1090,33 @@ extern "C" int pt_adamw_step_dev(float* p, const void* g, int g_is_bf16, float* 
   PT_REQUIRE(n > 0 && n % 4 == 0, "adamw_step_dev: n=%lld must be a positive multiple of 4", (long long)n);
   PT_REQUIRE(p && g && m && v && state, "adamw_step_dev: null pointer");
   if (g_is_bf16)
-    adamw_dev_kernel<true><<<grid_for(n / 4, 1024, 4), 256, 0, ST>>>(p, g, m, v, (bf16*)w_bf16, n / 4, state);
+    adamw_dev_kernel<true, false><<<grid_for(n / 4, 1024, 4), 256, 0, ST>>>(p, g, m, v, (bf16*)w_bf16, n / 4, state, nullptr, nullptr);
   else
-    adamw_dev_kernel<false><<<grid_for(n / 4, 1024, 4), 256, 0, ST>>>(p, g, m, v, (bf16*)w_bf16, n / 4, state);
+    adamw_dev_kernel<false, false><<<grid_for(n / 4, 1024, 4), 256, 0, ST>>>(p, g, m, v, (bf16*)w_bf16, n / 4, state, nullptr, nullptr);
+  PT_LAUNCH_CHECK();
+  return PT_OK;
+}
+extern "C" int pt_ema_prepare(double* ema_state, void* stream) {
+  PT_REQUIRE(ema_state != nullptr, "ema_prepare: null state");
+  ema_prepare_kernel<<<1, 1, 0, ST>>>(ema_state);
+  PT_LAUNCH_CHECK();
+  return PT_OK;
+}
+extern "C" int pt_adamw_ema_step_dev(float* p, const void* g, int g_is_bf16, float* m, float* v, void* w_bf16, float* ema, int64_t n,
+                                     const float* state, const double* ema_state, void* stream) {
+  PT_REQUIRE(n > 0 && n % 4 == 0, "adamw_ema_step_dev: n=%lld must be a positive multiple of 4", (long long)n);
+  PT_REQUIRE(p && g && m && v && ema && state && ema_state, "adamw_ema_step_dev: null pointer");
+  if (g_is_bf16)
+    adamw_dev_kernel<true, true><<<grid_for(n / 4, 1024, 4), 256, 0, ST>>>(p, g, m, v, (bf16*)w_bf16, n / 4, state, ema, ema_state);
+  else
+    adamw_dev_kernel<false, true><<<grid_for(n / 4, 1024, 4), 256, 0, ST>>>(p, g, m, v, (bf16*)w_bf16, n / 4, state, ema, ema_state);
+  PT_LAUNCH_CHECK();
+  return PT_OK;
+}
+extern "C" int pt_ema_swap(float* p, float* ema, void* w_bf16, int64_t n, void* stream) {
+  PT_REQUIRE(n > 0 && n % 4 == 0, "ema_swap: n=%lld must be a positive multiple of 4", (long long)n);
+  PT_REQUIRE(p && ema && w_bf16, "ema_swap: null pointer");
+  ema_swap_kernel<<<grid_for(n / 4, 1024, 4), 256, 0, ST>>>((float4*)p, (float4*)ema, (uint2*)w_bf16, n / 4);
   PT_LAUNCH_CHECK();
   return PT_OK;
 }
