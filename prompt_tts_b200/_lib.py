@@ -125,9 +125,13 @@ _SIGS = {
     "text_embed_bwd": "pppiiiip",
     "add_noise": "ppppppilp",
     "mse_fwd_bwd": "pppplfp",
+    "diffusion_loss": "ppppppppiliffp",
     "ddpm_step": "pppppliiffp",
     "ddim_step": "ppppppliifffffp",
     "dpmpp_step": "pppppppliifffiffp",
+    "ddpm_step_pred": "pppppliiffip",
+    "ddim_step_pred": "ppppppliifffffip",
+    "dpmpp_step_pred": "pppppppliifffiffip",
     "cond_select_bf16": "pppilp",
     "cfg_combine": "pplfp",
     "rows_add_bias_bf16": "ppplip",

@@ -3,6 +3,8 @@ only as device-memory handles; every computation below is a hand-written sm_100a
 from __future__ import annotations
 
 import ctypes as C
+import math
+import numbers
 from typing import Optional, Sequence
 
 import torch
@@ -20,6 +22,20 @@ def _stream() -> C.c_void_p:
 
 def _p(t: Optional[torch.Tensor]) -> C.c_void_p:
     return C.c_void_p(0 if t is None else t.data_ptr())
+
+
+# diffusers' scheduler `prediction_type` -> PT_PRED_* of the header
+PRED_TYPES = {"epsilon": 0, "sample": 1, "v_prediction": 2}
+
+
+def check_prediction(name: str, prediction_type, snr_gamma=None):
+    """Validate a `prediction_type` / `snr_gamma` pair before any device work; returns (PT_PRED_* code, gamma with 0 = off)."""
+    if not isinstance(prediction_type, str) or prediction_type not in PRED_TYPES:
+        raise ValueError(f"{name}: prediction_type must be one of {sorted(PRED_TYPES)}, got {prediction_type!r}")
+    if snr_gamma is not None and (isinstance(snr_gamma, bool) or not isinstance(snr_gamma, numbers.Real)
+                                  or not math.isfinite(float(snr_gamma)) or float(snr_gamma) <= 0.0):
+        raise ValueError(f"{name}: snr_gamma must be None (no Min-SNR weighting) or a finite real number > 0, got {snr_gamma!r}")
+    return PRED_TYPES[prediction_type], (0.0 if snr_gamma is None else float(snr_gamma))
 
 
 def _need(t: torch.Tensor, dtype, what: str):

@@ -24,6 +24,12 @@ step runs the denoiser once at batch 2B -- rows [0, B) conditioned on the text, 
 context, what condition dropout trains: `DenoiserTrainStep(..., cond_keep=)`) -- and the step uses
 eps = eps_u + w (eps_c - eps_u) (`pt_cfg_combine`).  The null rows' cross-attention is exactly to_out's bias added to the residual
 (ldm/attention.py:BasicTransformerBlock._cross_guided), so it is computed as that.  w = 1 (the default) is the unguided loop.
+
+Prediction type (all three samplers, keyword `prediction_type`, as diffusers' schedulers take it): the model output is eps
+("epsilon", the default, the reference's), x0 ("sample") or v ("v_prediction"), matching what the model was trained to predict
+(`DenoiserTrainStep(..., prediction_type=)`).  The default calls `pt_ddpm_step` / `pt_ddim_step` / `pt_dpmpp_step`; the other types
+call their `_pred` variants, which convert the output as diffusers 0.15's `step` does inside the same single pass.  Guidance combines
+the raw outputs whatever they parameterise, as diffusers' pipelines do.
 """
 from __future__ import annotations
 
@@ -54,7 +60,9 @@ class _Sampler:
     call 1 and replayed; `_step` is the scheduler's update of x in place from the eps the forward left in `_static["eps"]`."""
     timesteps: List[int]
 
-    def __init__(self, model, n_infer: int, use_graph: bool):
+    def __init__(self, model, n_infer: int, use_graph: bool, prediction_type: str):
+        self.pred_type, _ = ops.check_prediction(type(self).__name__, prediction_type)
+        self.prediction_type = prediction_type
         self.model = model
         self.n_infer = n_infer
         self.acp = ddpm_alphas_cumprod()                      # host copy: the step coefficients are scalars per step
@@ -86,6 +94,13 @@ class _Sampler:
 
     def _step(self, i: int, t: int, x: torch.Tensor, noises: Optional[torch.Tensor], gen: torch.Generator) -> None:
         raise NotImplementedError
+
+    def _step_call(self, name: str, *args) -> None:
+        """the scheduler's step kernel: `pt_<name>` for epsilon prediction, `pt_<name>_pred` for the other types"""
+        if self.pred_type == 0:
+            ops.call(name, *args, ops._stream())
+        else:
+            ops.call(name + "_pred", *args, self.pred_type, ops._stream())
 
     @torch.no_grad()
     def sample(self, ids: torch.Tensor, T: int, x_T: Optional[torch.Tensor] = None, noises: Optional[torch.Tensor] = None,
@@ -156,8 +171,8 @@ class _Sampler:
 
 
 class DDPMSampler(_Sampler):
-    def __init__(self, model, n_infer: int = 100, n_train: int = 1000, use_graph: bool = True):
-        super().__init__(model, n_infer, use_graph)
+    def __init__(self, model, n_infer: int = 100, n_train: int = 1000, use_graph: bool = True, *, prediction_type: str = "epsilon"):
+        super().__init__(model, n_infer, use_graph, prediction_type)
         self.n_train = n_train
         self.stride = n_train // n_infer
         self.acp = ddpm_alphas_cumprod(n_train)
@@ -182,8 +197,8 @@ class DDPMSampler(_Sampler):
             # in-paint: the prompt frames of x_{t_prev} are the clean prompt noised to level t_prev (clean at the last step)
             sa, sb = (acp_prev ** 0.5, (1.0 - acp_prev) ** 0.5) if t_prev >= 0 else (1.0, 0.0)
             known[..., :keep] = sa * self._prompt + sb * self._prompt_noise[i]
-        ops.call("ddpm_step", ops._p(self._static["eps"]), ops._p(x), ops._p(noise if t_prev >= 0 else None), ops._p(known), ops._p(x),
-                 x.numel(), self._T, keep, acp_t, acp_prev, ops._stream())
+        self._step_call("ddpm_step", ops._p(self._static["eps"]), ops._p(x), ops._p(noise if t_prev >= 0 else None), ops._p(known),
+                        ops._p(x), x.numel(), self._T, keep, acp_t, acp_prev)
 
 
 def _check_steps(name: str, n_infer, hi: int) -> int:
@@ -221,11 +236,11 @@ class DDIMSampler(_KernelPromptSampler):
     """diffusers 0.15 `DDIMScheduler` (clip_sample, set_alpha_to_one, steps_offset 0) over the training schedule: timesteps
     (n_infer - 1) * r, ..., r, 0 with r = 1000 // n_infer.  eta = 0 is deterministic; eta = 1 adds the DDPM posterior's noise."""
 
-    def __init__(self, model, n_infer: int = 50, eta: float = 0.0, use_graph: bool = True):
+    def __init__(self, model, n_infer: int = 50, eta: float = 0.0, use_graph: bool = True, *, prediction_type: str = "epsilon"):
         n_infer = _check_steps("DDIMSampler", n_infer, 1000)
         if not 0.0 <= eta <= 1.0:
             raise ValueError(f"DDIMSampler: eta must be in [0, 1] (DDIM's interpolation between deterministic and DDPM noise), got {eta!r}")
-        super().__init__(model, n_infer, use_graph)
+        super().__init__(model, n_infer, use_graph, prediction_type)
         self.eta = float(eta)
         self.stride = 1000 // n_infer
         self.timesteps = [i * self.stride for i in range(n_infer)][::-1]
@@ -243,8 +258,8 @@ class DDIMSampler(_KernelPromptSampler):
             else:
                 self._noise.normal_(generator=gen)
         pp, pn, pa, pb = self._prompt_args(i, acp_prev if t_prev >= 0 else None)
-        ops.call("ddim_step", ops._p(self._static["eps"]), ops._p(x), ops._p(self._noise), pp, pn, ops._p(x), x.numel(), x.shape[-1], self._keep,
-                 float(self.acp[t]), acp_prev, self.eta, pa, pb, ops._stream())
+        self._step_call("ddim_step", ops._p(self._static["eps"]), ops._p(x), ops._p(self._noise), pp, pn, ops._p(x), x.numel(), x.shape[-1],
+                        self._keep, float(self.acp[t]), acp_prev, self.eta, pa, pb)
 
 
 class DPMSolverSampler(_KernelPromptSampler):
@@ -253,9 +268,9 @@ class DPMSolverSampler(_KernelPromptSampler):
     last one when n_infer < 15), second order from the x0 prediction of the previous step otherwise.  n_infer <= 999: at 1000 the
     rounded grid repeats a timestep."""
 
-    def __init__(self, model, n_infer: int = 20, use_graph: bool = True):
+    def __init__(self, model, n_infer: int = 20, use_graph: bool = True, *, prediction_type: str = "epsilon"):
         n_infer = _check_steps("DPMSolverSampler", n_infer, 999)
-        super().__init__(model, n_infer, use_graph)
+        super().__init__(model, n_infer, use_graph, prediction_type)
         self.timesteps = np.linspace(0, 999, n_infer + 1).round()[::-1][:-1].astype(np.int64).tolist()
 
     def _start(self, x, prompt, prompt_noise, keep):
@@ -269,5 +284,5 @@ class DPMSolverSampler(_KernelPromptSampler):
         order = 1 if i == 0 or (last and n < 15) else 2
         acp_s1 = float(self.acp[self.timesteps[i - 1]]) if order == 2 else 0.0
         pp, pn, pa, pb = self._prompt_args(i, None if last else float(self.acp[t_to]))
-        ops.call("dpmpp_step", ops._p(self._static["eps"]), ops._p(x), ops._p(self._m), ops._p(self._m), pp, pn, ops._p(x), x.numel(),
-                 x.shape[-1], self._keep, float(self.acp[t]), acp_s1, float(self.acp[t_to]), order, pa, pb, ops._stream())
+        self._step_call("dpmpp_step", ops._p(self._static["eps"]), ops._p(x), ops._p(self._m), ops._p(self._m), pp, pn, ops._p(x), x.numel(),
+                        x.shape[-1], self._keep, float(self.acp[t]), acp_s1, float(self.acp[t_to]), order, pa, pb)

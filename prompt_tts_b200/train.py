@@ -12,6 +12,12 @@ the reference's logical shapes), so the reference's `clip_grad_norm_` / `AdamW` 
 Classifier-free guidance training (not in the reference tree): `cond_keep` (bool [B]) replaces the text encoding of the samples
 where it is False with the null condition, an all-zero context, before the denoiser sees it (condition dropout).  The caller draws
 the mask each step, e.g. `torch.rand(B, device=dev) >= p_uncond`, as it draws `noise` and `t`.
+
+Prediction type and Min-SNR weighting (not in the reference tree, which trains epsilon prediction): with
+`DenoiserTrainStep(..., prediction_type="v_prediction" | "sample")` the loss target is diffusers' `get_velocity(x0, noise, t)` or
+x0 instead of `noise`, and `snr_gamma=g` weights each sample's MSE by Min-SNR-g (`compute_snr` of diffusers' training examples:
+min(snr, g) / snr for epsilon, / (snr + 1) for v, min(snr, g) for sample).  The target and the weight are formed inside one kernel
+(`pt_diffusion_loss`), from `t` on the device.  The samplers must be built with the same `prediction_type`.
 """
 from __future__ import annotations
 
@@ -31,13 +37,18 @@ def ddpm_tables(n: int = 1000, beta_start: float = 1e-4, beta_end: float = 0.02,
 
 
 class DenoiserTrainStep:
-    def __init__(self, model, grad_sync=None, accumulation_steps: int = 1):
+    def __init__(self, model, grad_sync=None, accumulation_steps: int = 1, *, prediction_type: str = "epsilon",
+                 snr_gamma: Optional[float] = None):
         """grad_sync: a `prompt_tts_b200.dp.GradSync` (flat gradient buffer; overlaps the gradient all-reduce with the backward
         sweep when world_size > 1); built for a single process when omitted.
         accumulation_steps: the reference's `gradient_accumulation_steps` (train.py:27,80 `accelerator.accumulate`): every call is
         one micro-step; the flat gradient buffer is cleared at the first micro-step of a window, the loss gradient is scaled by
         1 / accumulation_steps (what `accelerator.backward` does), ranks exchange gradients only during the last micro-step, and
-        `sync_gradients` tells the optimiser wrapper whether to step (`FusedClipAdamW.step` is a no-op otherwise)."""
+        `sync_gradients` tells the optimiser wrapper whether to step (`FusedClipAdamW.step` is a no-op otherwise).
+        prediction_type: "epsilon" (the reference's), "sample" or "v_prediction" -- diffusers' scheduler option of that name.
+        snr_gamma: None (unweighted, the reference's) or gamma > 0 of Min-SNR-gamma loss weighting (module docstring)."""
+        self.pred_type, self._snr_gamma = ops.check_prediction("DenoiserTrainStep", prediction_type, snr_gamma)
+        self.prediction_type = prediction_type
         self.model = model
         self.params = [p for p in model.parameters()]
         self.cache = E.get_cache(model)
@@ -97,7 +108,12 @@ class DenoiserTrainStep:
         pred, seed = self.model.unet._fwd(tape, xt, t, enc)
         loss = torch.zeros((), dtype=torch.float32, device=x0.device) if loss_out is None else loss_out.zero_()
         dpred = torch.empty_like(pred)
-        ops.call("mse_fwd_bwd", ops._p(pred), ops._p(noise), ops._p(loss), ops._p(dpred), pred.numel(), gscale / self.accumulation_steps, ops._stream())
+        gs = gscale / self.accumulation_steps
+        if self.pred_type == 0 and self._snr_gamma == 0.0:
+            ops.call("mse_fwd_bwd", ops._p(pred), ops._p(noise), ops._p(loss), ops._p(dpred), pred.numel(), gs, ops._stream())
+        else:
+            ops.call("diffusion_loss", ops._p(pred), ops._p(x0), ops._p(noise), ops._p(t), ops._p(self.sa), ops._p(self.sb), ops._p(loss),
+                     ops._p(dpred), B, x0[0].numel(), self.pred_type, self._snr_gamma, gs, ops._stream())
         seed([dpred])
         tape.backward()
         self.grad_sync.finish()
