@@ -27,9 +27,9 @@ eps = eps_u + w (eps_c - eps_u) (`pt_cfg_combine`).  The null rows' cross-attent
 
 Prediction type (all three samplers, keyword `prediction_type`, as diffusers' schedulers take it): the model output is eps
 ("epsilon", the default, the reference's), x0 ("sample") or v ("v_prediction"), matching what the model was trained to predict
-(`DenoiserTrainStep(..., prediction_type=)`).  The default calls `pt_ddpm_step` / `pt_ddim_step` / `pt_dpmpp_step`; the other types
-call their `_pred` variants, which convert the output as diffusers 0.15's `step` does inside the same single pass.  Guidance combines
-the raw outputs whatever they parameterise, as diffusers' pipelines do.
+(`DenoiserTrainStep(..., prediction_type=)`).  Every type calls the `_pred` step entry points with the type; they convert the output
+as diffusers 0.15's `step` does inside the same single pass.  Guidance combines the raw outputs whatever they parameterise, as
+diffusers' pipelines do.
 """
 from __future__ import annotations
 
@@ -96,11 +96,15 @@ class _Sampler:
         raise NotImplementedError
 
     def _step_call(self, name: str, *args) -> None:
-        """the scheduler's step kernel: `pt_<name>` for epsilon prediction, `pt_<name>_pred` for the other types"""
-        if self.pred_type == 0:
-            ops.call(name, *args, ops._stream())
+        """the scheduler's step kernel `pt_<name>_pred` for the model's prediction type"""
+        ops.call(name + "_pred", *args, self.pred_type, ops._stream())
+
+    def _draw_noise(self, i: int, noises: Optional[torch.Tensor], gen: torch.Generator) -> None:
+        """the step's noise buffer: noises[i] when given, else a draw from the sampler's generator"""
+        if noises is not None:
+            self._noise.copy_(noises[i])
         else:
-            ops.call(name + "_pred", *args, self.pred_type, ops._stream())
+            self._noise.normal_(generator=gen)
 
     @torch.no_grad()
     def sample(self, ids: torch.Tensor, T: int, x_T: Optional[torch.Tensor] = None, noises: Optional[torch.Tensor] = None,
@@ -172,6 +176,7 @@ class _Sampler:
 
 class DDPMSampler(_Sampler):
     def __init__(self, model, n_infer: int = 100, n_train: int = 1000, use_graph: bool = True, *, prediction_type: str = "epsilon"):
+        n_infer = _check_steps("DDPMSampler", n_infer, n_train)
         super().__init__(model, n_infer, use_graph, prediction_type)
         self.n_train = n_train
         self.stride = n_train // n_infer
@@ -189,10 +194,7 @@ class DDPMSampler(_Sampler):
         acp_t = float(self.acp[t])
         acp_prev = float(self.acp[t_prev]) if t_prev >= 0 else 1.0
         if t_prev >= 0:
-            if noises is not None:
-                noise.copy_(noises[i])
-            else:
-                noise.normal_(generator=gen)
+            self._draw_noise(i, noises, gen)
         if known is not None:
             # in-paint: the prompt frames of x_{t_prev} are the clean prompt noised to level t_prev (clean at the last step)
             sa, sb = (acp_prev ** 0.5, (1.0 - acp_prev) ** 0.5) if t_prev >= 0 else (1.0, 0.0)
@@ -253,10 +255,7 @@ class DDIMSampler(_KernelPromptSampler):
         t_prev = t - self.stride
         acp_prev = float(self.acp[t_prev]) if t_prev >= 0 else 1.0
         if self._noise is not None:
-            if noises is not None:
-                self._noise.copy_(noises[i])
-            else:
-                self._noise.normal_(generator=gen)
+            self._draw_noise(i, noises, gen)
         pp, pn, pa, pb = self._prompt_args(i, acp_prev if t_prev >= 0 else None)
         self._step_call("ddim_step", ops._p(self._static["eps"]), ops._p(x), ops._p(self._noise), pp, pn, ops._p(x), x.numel(), x.shape[-1],
                         self._keep, float(self.acp[t]), acp_prev, self.eta, pa, pb)

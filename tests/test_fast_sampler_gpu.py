@@ -7,7 +7,8 @@ import sys
 import pytest
 import torch
 
-from util import ROOT, load_cfg, rel, synth_inputs
+import sampling_oracle as so
+from util import ROOT, rel, synth_inputs
 
 sys.path.insert(0, os.path.join(ROOT, "oracle", "diffusers_shim"))
 from diffusers.schedulers_few_step import DDIMScheduler, DPMSolverMultistepScheduler  # noqa: E402
@@ -107,54 +108,9 @@ def test_step_kernels_inpaint_prompt_frames(cuda):
 SAMPLERS = [("ddim", 0.0), ("ddim", 1.0), ("dpm", None)]
 
 
-def _sampler(model, kind, eta, n_infer, use_graph=True):
-    from prompt_tts_b200.sample import DDIMSampler, DPMSolverSampler
-    if kind == "ddim":
-        return DDIMSampler(model, n_infer=n_infer, eta=eta, use_graph=use_graph)
-    return DPMSolverSampler(model, n_infer=n_infer, use_graph=use_graph)
-
-
-def _oracle_loop(model, cfg, kind, eta, n_infer, ids, x_T, noises, prompt=None, prompt_noise=None, toks=None, eps_err=0.0):
-    """fp32 reference denoiser + the shim scheduler; prompt frames overwritten after every step with the prompt noised to the
-    level the step landed on (clean after the last step).  eps_err > 0 adds seeded Gaussian noise of that relative size to every
-    denoiser output: how far the loop itself carries a given per-call error."""
-    import ref_model
-    sched = DDIMScheduler() if kind == "ddim" else DPMSolverMultistepScheduler()
-    sched.set_timesteps(n_infer)
-    ts = sched.timesteps.tolist()
-    acp = sched.alphas_cumprod
-    sd = {k: v.detach().float() for k, v in model.state_dict().items()}
-    B = x_T.shape[0]
-    g = torch.Generator(device=x_T.device).manual_seed(17)
-    with torch.no_grad():
-        enc = ref_model.text_encoder(sd, cfg, ids)
-        if toks is not None:
-            enc = torch.cat([enc, toks], dim=1)
-        x = x_T.clone()
-        for i, t in enumerate(ts):
-            eps = ref_model.unet(sd, cfg, x, torch.full((B,), t, device=x.device, dtype=torch.int64), enc)
-            if eps_err > 0:
-                eps = eps + eps_err * eps.norm() / eps.numel() ** 0.5 * torch.randn(eps.shape, device=eps.device, generator=g)
-            if kind == "ddim":
-                x = sched.step(eps, t, x, eta=eta, variance_noise=noises[i]).prev_sample
-            else:
-                x = sched.step(eps, t, x).prev_sample
-            if prompt is not None:
-                to = (t - 1000 // n_infer if kind == "ddim" else (ts[i + 1] if i + 1 < n_infer else -1))
-                keep = prompt.shape[-1]
-                if i == n_infer - 1 or to < 0:
-                    x[..., :keep] = prompt
-                else:
-                    x[..., :keep] = acp[to].sqrt() * prompt + (1 - acp[to]).sqrt() * prompt_noise[i]
-    return x
-
-
 @pytest.fixture(scope="module")
 def tiny(cuda):
-    from prompt_tts_b200.models import TTSSingleSpeaker
-    cfg = load_cfg("tiny")
-    torch.manual_seed(0)
-    return cfg, TTSSingleSpeaker(cfg).to(cuda).eval()
+    return so.load_model("tiny", cuda)
 
 
 @pytest.mark.parametrize("kind,eta", SAMPLERS)
@@ -165,10 +121,11 @@ def test_fast_sampler_matches_oracle_loop(cuda, tiny, kind, eta):
     g = torch.Generator(device="cuda").manual_seed(9)
     x_T = torch.randn(B, cfg["in_channels"], T, device=cuda, generator=g)
     noises = torch.randn(n_infer, B, cfg["in_channels"], T, device=cuda, generator=g)
-    outs = {graph: _sampler(model, kind, eta, n_infer, graph).sample(inp["ids"], T, x_T=x_T, noises=noises) for graph in (False, True)}
+    outs = {graph: so.make_sampler(model, kind, eta, n_infer, use_graph=graph).sample(inp["ids"], T, x_T=x_T, noises=noises)
+            for graph in (False, True)}
     # GroupNorm statistics are accumulated with fp32 atomics (order not fixed), so two runs agree to rounding, not bit for bit
     assert rel(outs[False], outs[True]) < 1e-3, "graph replay must reproduce the eager loop"
-    x = _oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises)
+    x = so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises)
     e = rel(outs[True], x)
     bound = 2e-2 * 2                # bf16 denoiser error (<= 2e-2 per call) carried through the steps; the step kernels are exact
     if kind == "ddim" and eta == 0.0:
@@ -177,7 +134,7 @@ def test_fast_sampler_matches_oracle_loop(cuda, tiny, kind, eta):
         # step, and no fresh noise dilutes it.  The fp32 oracle loop alone turns a 1e-2 random per-call error into 8e-2 at the
         # output here (DDPM 0.7e-2, eta = 1 1.1e-2, DPM-Solver++ 0.35e-2); the product (6.2e-2) is held to what the oracle loop
         # makes of the per-call bar of 2e-2.
-        bound = rel(_oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, eps_err=2e-2), x)
+        bound = rel(so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, eps_err=2e-2, err_seed=17), x)
     print(f"\n[{kind} eta={eta} tiny, {n_infer} steps] rel err vs fp32 oracle loop {e:.2e} (bound {bound:.2e})")
     assert e < bound, (e, bound)
 
@@ -188,7 +145,7 @@ def test_fast_sampler_prompt_inpainting_and_codes(cuda, tiny, kind, eta):
     B, T, P, n_infer = 2, 16, 6, 4
     inp = synth_inputs(cfg, B, T, seed=6, device=cuda)
     prompt = inp["x0"][..., :P].contiguous()
-    smp = _sampler(model, kind, eta, n_infer)
+    smp = so.make_sampler(model, kind, eta, n_infer)
     x = smp.sample(inp["ids"], T, prompt=prompt, seed=3)
     assert torch.equal(x[..., :P], prompt), "the prompt frames must come out clean"
     assert torch.isfinite(x).all()
@@ -202,7 +159,7 @@ def test_fast_sampler_prompt_inpainting_and_codes(cuda, tiny, kind, eta):
     noises = torch.randn(n_infer, B, cfg["in_channels"], T, device=cuda, generator=g)
     pn = torch.randn(n_infer, B, cfg["in_channels"], P, device=cuda, generator=g)
     got = smp.sample(inp["ids"], T, x_T=x_T, noises=noises, prompt=prompt, prompt_noise=pn)
-    want = _oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, prompt, pn)
+    want = so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, prompt=prompt, prompt_noise=pn)
     assert torch.equal(got[..., :P], want[..., :P])
     assert rel(got, want) < 4e-2, rel(got, want)
     with pytest.raises(Exception, match="prompt must be"):
@@ -220,9 +177,9 @@ def test_fast_sampler_prompt_tokens(cuda, tiny, kind, eta):
     x_T = torch.randn(B, cfg["in_channels"], T, device=cuda, generator=g)
     noises = torch.randn(n_infer, B, cfg["in_channels"], T, device=cuda, generator=g)
     toks = torch.randn(B, P, cfg["cross_attention_dim"], device=cuda, generator=g)
-    smp = _sampler(model, kind, eta, n_infer)
+    smp = so.make_sampler(model, kind, eta, n_infer)
     with_t = smp.sample(inp["ids"], T, x_T=x_T, noises=noises, prompt_tokens=toks)
     without = smp.sample(inp["ids"], T, x_T=x_T, noises=noises)
     assert rel(with_t, without) > 1e-3
-    x = _oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, toks=toks)
+    x = so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, toks=toks)
     assert rel(with_t, x) < 4e-2, rel(with_t, x)

@@ -3,27 +3,14 @@ block bit for bit against the product's own unguided block, one guided denoiser 
 loops against an fp32 oracle (oracle/ref_model.py denoiser on the text encoding and on zeros, eps_u + w (eps_c - eps_u), the
 shim's step), and condition dropout in the train step and in TTSSingleSpeaker.forward against the oracle with the text encoding
 selected by the keep mask."""
-import os
-import sys
-
 import pytest
 import torch
 
-from util import ROOT, load_cfg, rel, synth_inputs
-
-sys.path.insert(0, os.path.join(ROOT, "oracle", "diffusers_shim"))
-from diffusers.schedulers_few_step import DDIMScheduler, DPMSolverMultistepScheduler  # noqa: E402
+import sampling_oracle as so
+from util import rel, synth_inputs
 
 pytestmark = pytest.mark.gpu
 TOL = 2e-2
-
-
-def _model(cfg_name, dev, train=False):
-    from prompt_tts_b200.models import TTSSingleSpeaker
-    cfg = load_cfg(cfg_name)
-    torch.manual_seed(0)
-    m = TTSSingleSpeaker(cfg).to(dev)
-    return cfg, (m if train else m.eval())
 
 
 # ---------------------------------------------------------------------------------------------------------------- kernels
@@ -124,7 +111,7 @@ def test_block_null_context_shortcut_is_exact(cuda, dim, ctx, Lk, B):
 def test_guided_forward_matches_oracle(cuda, cfg_name):
     import ref_model
     from prompt_tts_b200 import engine as E
-    cfg, model = _model(cfg_name, cuda)
+    cfg, model = so.load_model(cfg_name, cuda)
     B, T = 1, 752
     inp = synth_inputs(cfg, B, T, seed=4, device=cuda)
     x = inp["noise"]
@@ -149,89 +136,26 @@ def test_guided_forward_matches_oracle(cuda, cfg_name):
 KINDS = [("ddpm", None), ("ddim", 0.0), ("ddim", 1.0), ("dpm", None)]
 
 
-def _sampler(model, kind, eta, n_infer, use_graph=True):
-    from prompt_tts_b200.sample import DDIMSampler, DDPMSampler, DPMSolverSampler
-    if kind == "ddpm":
-        return DDPMSampler(model, n_infer=n_infer, use_graph=use_graph)
-    if kind == "ddim":
-        return DDIMSampler(model, n_infer=n_infer, eta=eta, use_graph=use_graph)
-    return DPMSolverSampler(model, n_infer=n_infer, use_graph=use_graph)
-
-
-def _oracle_loop(model, cfg, kind, eta, n_infer, w, ids, x_T, noises, prompt=None, prompt_noise=None, eps_err=0.0):
-    """fp32 guided loop: ref_model.text_encoder once, ref_model.unet on the encoding and on zeros, eps_u + w (eps_c - eps_u),
-    the scheduler's step; prompt frames overwritten after every step with the prompt noised to the level the step landed on.
-    eps_err > 0 adds a seeded Gaussian error of that relative size to each of eps_c and eps_u: what the loop itself makes of a
-    given per-call error of the denoiser."""
-    import ref_model
-    acp = ref_model.ddpm_alphas_cumprod().to(x_T.device)
-    if kind == "ddpm":
-        ts = [k * (1000 // n_infer) for k in range(n_infer)][::-1]
-    else:
-        sched = DDIMScheduler() if kind == "ddim" else DPMSolverMultistepScheduler()
-        sched.set_timesteps(n_infer)
-        ts = sched.timesteps.tolist()
-    sd = {k: v.detach().float() for k, v in model.state_dict().items()}
-    B = x_T.shape[0]
-    g = torch.Generator(device=x_T.device).manual_seed(23)
-
-    def err(e):
-        return e + eps_err * e.norm() / e.numel() ** 0.5 * torch.randn(e.shape, device=e.device, generator=g) if eps_err > 0 else e
-
-    with torch.no_grad():
-        enc = ref_model.text_encoder(sd, cfg, ids)
-        x = x_T.clone()
-        for i, t in enumerate(ts):
-            tt = torch.full((B,), t, device=x.device, dtype=torch.int64)
-            c = err(ref_model.unet(sd, cfg, x, tt, enc))
-            u = err(ref_model.unet(sd, cfg, x, tt, torch.zeros_like(enc)))
-            eps = u + w * (c - u)
-            if kind == "ddpm":
-                x = ref_model.ddpm_step(eps, t, x, noises[i], acp=acp, n_infer=n_infer)
-                to = t - 1000 // n_infer
-            elif kind == "ddim":
-                x = sched.step(eps, t, x, eta=eta, variance_noise=noises[i]).prev_sample
-                to = t - 1000 // n_infer
-            else:
-                x = sched.step(eps, t, x).prev_sample
-                to = ts[i + 1] if i + 1 < n_infer else -1
-            if prompt is not None:
-                keep = prompt.shape[-1]
-                if i == n_infer - 1 or to < 0:
-                    x[..., :keep] = prompt
-                else:
-                    x[..., :keep] = acp[to].sqrt() * prompt + (1 - acp[to]).sqrt() * prompt_noise[i]
-    return x
-
-
 @pytest.fixture(scope="module")
 def tiny(cuda):
-    return _model("tiny", cuda)
-
-
-def _case(cfg, B, T, n_infer, seed, dev):
-    inp = synth_inputs(cfg, B, T, seed=seed, device=dev)
-    g = torch.Generator(device="cuda").manual_seed(seed + 100)
-    x_T = torch.randn(B, cfg["in_channels"], T, device=dev, generator=g)
-    noises = torch.randn(n_infer, B, cfg["in_channels"], T, device=dev, generator=g)
-    return inp, x_T, noises
+    return so.load_model("tiny", cuda)
 
 
 @pytest.mark.parametrize("kind,eta", KINDS)
 def test_guided_loop_matches_oracle(cuda, tiny, kind, eta):
     cfg, model = tiny
     B, T, n_infer, w = 2, 16, 5, 3.0
-    inp, x_T, noises = _case(cfg, B, T, n_infer, 5, cuda)
-    outs = {gr: _sampler(model, kind, eta, n_infer, gr).sample(inp["ids"], T, x_T=x_T, noises=noises, guidance_scale=w)
+    inp, x_T, noises = so.case(cfg, B, T, n_infer, 5, cuda)
+    outs = {gr: so.make_sampler(model, kind, eta, n_infer, use_graph=gr).sample(inp["ids"], T, x_T=x_T, noises=noises, guidance_scale=w)
             for gr in (False, True)}
     assert outs[True].shape == x_T.shape and outs[True].is_contiguous()
     # GroupNorm statistics are accumulated with fp32 atomics (order not fixed), so two runs agree to rounding, not bit for bit
     assert rel(outs[False], outs[True]) < 1e-3, "graph replay must reproduce the eager loop"
-    x = _oracle_loop(model, cfg, kind, eta, n_infer, w, inp["ids"], x_T, noises)
-    unguided = _oracle_loop(model, cfg, kind, eta, n_infer, 1.0, inp["ids"], x_T, noises)
+    x = so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, w=w)
+    unguided = so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, w=1.0)
     # guidance multiplies a per-call error of the denoiser by about w: the bar is what the fp32 oracle loop makes of the 2e-2
     # per-call bar on each of eps_c and eps_u
-    bound = rel(_oracle_loop(model, cfg, kind, eta, n_infer, w, inp["ids"], x_T, noises, eps_err=TOL), x)
+    bound = rel(so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, w=w, eps_err=TOL, err_seed=23), x)
     e = {gr: rel(outs[gr], x) for gr in (False, True)}
     print(f"\n[guided {kind} eta={eta} tiny w={w}, {n_infer} steps] rel err vs fp32 oracle loop: graph {e[True]:.2e}, eager "
           f"{e[False]:.2e} (bound {bound:.2e}; guided vs unguided oracle {rel(x, unguided):.2e})")
@@ -242,9 +166,9 @@ def test_guided_loop_matches_oracle(cuda, tiny, kind, eta):
 def test_guided_loop_prompt_and_codes(cuda, tiny, kind, eta):
     cfg, model = tiny
     B, T, P, n_infer, w = 2, 16, 6, 4, 3.0
-    inp, x_T, noises = _case(cfg, B, T, n_infer, 6, cuda)
+    inp, x_T, noises = so.case(cfg, B, T, n_infer, 6, cuda)
     prompt = inp["x0"][..., :P].contiguous()
-    smp = _sampler(model, kind, eta, n_infer)
+    smp = so.make_sampler(model, kind, eta, n_infer)
     x = smp.sample(inp["ids"], T, prompt=prompt, seed=3, guidance_scale=w)
     assert torch.equal(x[..., :P], prompt), "the prompt frames must come out clean"
     assert torch.isfinite(x).all()
@@ -253,8 +177,9 @@ def test_guided_loop_prompt_and_codes(cuda, tiny, kind, eta):
     g = torch.Generator(device="cuda").manual_seed(12)
     pn = torch.randn(n_infer, B, cfg["in_channels"], P, device=cuda, generator=g)
     got = smp.sample(inp["ids"], T, x_T=x_T, noises=noises, prompt=prompt, prompt_noise=pn, guidance_scale=w)
-    want = _oracle_loop(model, cfg, kind, eta, n_infer, w, inp["ids"], x_T, noises, prompt, pn)
-    bound = rel(_oracle_loop(model, cfg, kind, eta, n_infer, w, inp["ids"], x_T, noises, prompt, pn, eps_err=TOL), want)
+    want = so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, w=w, prompt=prompt, prompt_noise=pn)
+    bound = rel(so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, w=w, prompt=prompt, prompt_noise=pn,
+                               eps_err=TOL, err_seed=23), want)
     print(f"\n[guided {kind} eta={eta} + prompt] rel err {rel(got, want):.2e} (bound {bound:.2e})")
     assert torch.equal(got[..., :P], want[..., :P])
     assert rel(got, want) < bound
@@ -264,10 +189,10 @@ def test_guided_loop_prompt_and_codes(cuda, tiny, kind, eta):
 def test_guided_loop_batch_one(cuda, tiny, kind, eta):
     cfg, model = tiny
     B, T, n_infer, w = 1, 32, 5, 4.0
-    inp, x_T, noises = _case(cfg, B, T, n_infer, 7, cuda)
-    got = _sampler(model, kind, eta, n_infer).sample(inp["ids"], T, x_T=x_T, noises=noises, guidance_scale=w)
-    want = _oracle_loop(model, cfg, kind, eta, n_infer, w, inp["ids"], x_T, noises)
-    bound = rel(_oracle_loop(model, cfg, kind, eta, n_infer, w, inp["ids"], x_T, noises, eps_err=TOL), want)
+    inp, x_T, noises = so.case(cfg, B, T, n_infer, 7, cuda)
+    got = so.make_sampler(model, kind, eta, n_infer).sample(inp["ids"], T, x_T=x_T, noises=noises, guidance_scale=w)
+    want = so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, w=w)
+    bound = rel(so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, w=w, eps_err=TOL, err_seed=23), want)
     print(f"\n[guided {kind} B=1 w={w}] rel err {rel(got, want):.2e} (bound {bound:.2e})")
     assert rel(got, want) < bound
 
@@ -276,9 +201,9 @@ def test_guided_loop_prompt_tokens(cuda, tiny):
     """prompt tokens extend the conditional rows' context only; the result differs from the text-only guided run"""
     cfg, model = tiny
     B, T, n_infer = 2, 16, 3
-    inp, x_T, noises = _case(cfg, B, T, n_infer, 8, cuda)
+    inp, x_T, noises = so.case(cfg, B, T, n_infer, 8, cuda)
     toks = torch.randn(B, 9, cfg["cross_attention_dim"], device=cuda)
-    smp = _sampler(model, "dpm", None, n_infer)
+    smp = so.make_sampler(model, "dpm", None, n_infer)
     a = smp.sample(inp["ids"], T, x_T=x_T, noises=noises, prompt_tokens=toks, guidance_scale=2.0)
     b = smp.sample(inp["ids"], T, x_T=x_T, noises=noises, guidance_scale=2.0)
     assert torch.isfinite(a).all() and rel(a, b) > 1e-3
@@ -289,8 +214,8 @@ def test_guidance_one_is_the_unguided_loop(cuda, tiny):
     from prompt_tts_b200 import _lib
     cfg, model = tiny
     B, T, n_infer = 2, 16, 4
-    inp, x_T, noises = _case(cfg, B, T, n_infer, 9, cuda)
-    smp = _sampler(model, "ddim", 0.0, n_infer)
+    inp, x_T, noises = so.case(cfg, B, T, n_infer, 9, cuda)
+    smp = so.make_sampler(model, "ddim", 0.0, n_infer)
     smp.sample(inp["ids"], T, x_T=x_T, noises=noises)          # first-use work (weight packs) outside the counted calls
     lib = _lib.lib()
     l0 = lib.pt_launch_count()
@@ -320,13 +245,6 @@ def _oracle_train(cfg, model, inp, keep):
     return xt, loss.detach(), {k: v.grad for k, v in sd.items() if v.requires_grad and v.grad is not None and v.grad.abs().max() > 0}
 
 
-def _grad_err(model, ref_grads):
-    named = dict(model.named_parameters())
-    keys = sorted(ref_grads)
-    assert all(named[k].grad is not None for k in keys), [k for k in keys if named[k].grad is None][:5]
-    return rel(torch.cat([named[k].grad.flatten() for k in keys]), torch.cat([ref_grads[k].flatten() for k in keys]))
-
-
 def _keep(B, dev):
     return (torch.arange(B, device=dev) % 3 != 1)          # mixed: 1, 0, 1, 1, 0, 1, ...
 
@@ -335,21 +253,21 @@ def _keep(B, dev):
 @pytest.mark.parametrize("cfg_name,B,T", [("tiny", 8, 64), ("tiny3", 8, 128), ("mid", 2, 64)])
 def test_train_step_condition_dropout_matches_oracle(cuda, cfg_name, B, T):
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = _model(cfg_name, cuda, train=True)
+    cfg, model = so.load_model(cfg_name, cuda, train=True)
     inp = synth_inputs(cfg, B, T, seed=1, device=cuda)
     keep = _keep(B, cuda)
     assert keep.any() and not keep.all()
     _, ref_loss, ref_grads = _oracle_train(cfg, model, inp, keep)
     loss = DenoiserTrainStep(model)(inp["x0"], inp["noise"], inp["t"], inp["ids"], inp["mask"], cond_keep=keep)
     torch.cuda.synchronize()
-    e_l, e_g = rel(loss, ref_loss), _grad_err(model, ref_grads)
+    e_l, e_g = rel(loss, ref_loss), so.grad_err(model, ref_grads)
     print(f"\n[{cfg_name} {B}x{T} condition dropout, keep {keep.int().tolist()}] loss {e_l:.2e} global grad {e_g:.2e}")
     assert e_l < TOL and e_g < TOL, (e_l, e_g)
 
 
 def test_train_step_all_dropped(cuda):
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = _model("tiny", cuda, train=True)
+    cfg, model = so.load_model("tiny", cuda, train=True)
     B, T = 8, 64
     inp = synth_inputs(cfg, B, T, seed=2, device=cuda)
     none = torch.zeros(B, dtype=torch.bool, device=cuda)
@@ -374,7 +292,7 @@ def test_train_step_all_dropped(cuda):
 
 def test_train_step_all_kept_is_the_default(cuda):
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = _model("tiny", cuda, train=True)
+    cfg, model = so.load_model("tiny", cuda, train=True)
     B, T = 8, 64
     inp = synth_inputs(cfg, B, T, seed=3, device=cuda)
     stepper = DenoiserTrainStep(model)
@@ -389,7 +307,7 @@ def test_train_step_all_kept_is_the_default(cuda):
 def test_train_step_graph_replays_fresh_masks(cuda):
     """a captured step reads the mask from its static buffer: replays with two masks equal eager steps with the same masks"""
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = _model("tiny", cuda, train=True)
+    cfg, model = so.load_model("tiny", cuda, train=True)
     B, T = 8, 64
     inp = synth_inputs(cfg, B, T, seed=4, device=cuda)
     stepper = DenoiserTrainStep(model)
@@ -426,7 +344,7 @@ def test_train_step_graph_replays_fresh_masks(cuda):
 
 
 def test_model_forward_cond_keep_matches_oracle(cuda):
-    cfg, model = _model("tiny", cuda, train=True)
+    cfg, model = so.load_model("tiny", cuda, train=True)
     B, T = 8, 64
     inp = synth_inputs(cfg, B, T, seed=5, device=cuda)
     keep = _keep(B, cuda)
@@ -435,7 +353,7 @@ def test_model_forward_cond_keep_matches_oracle(cuda):
     loss = torch.nn.functional.mse_loss(out, inp["noise"])
     loss.backward()
     torch.cuda.synchronize()
-    e_l, e_g = rel(loss, ref_loss), _grad_err(model, ref_grads)
+    e_l, e_g = rel(loss, ref_loss), so.grad_err(model, ref_grads)
     print(f"\n[TTSSingleSpeaker.forward cond_keep, tiny {B}x{T}] loss {e_l:.2e} global grad {e_g:.2e}")
     assert e_l < TOL and e_g < TOL, (e_l, e_g)
 
@@ -443,7 +361,7 @@ def test_model_forward_cond_keep_matches_oracle(cuda):
 def test_bad_cond_keep_raises(cuda):
     from prompt_tts_b200 import _lib
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = _model("tiny", cuda, train=True)
+    cfg, model = so.load_model("tiny", cuda, train=True)
     B, T = 2, 16
     inp = synth_inputs(cfg, B, T, seed=6, device=cuda)
     stepper = DenoiserTrainStep(model)

@@ -8,22 +8,15 @@ import pytest
 import torch
 
 import prediction_oracle as po
+import sampling_oracle as so
 from prediction_oracle import DDIMScheduler, DDPMScheduler, DPMSolverMultistepScheduler
-from util import load_cfg, rel, synth_inputs
+from util import rel, synth_inputs
 
 pytestmark = pytest.mark.gpu
 TOL = 2e-2
 PRED = {"epsilon": 0, "sample": 1, "v_prediction": 2}
 NON_EPS = ("sample", "v_prediction")
 SHAPE = (3, 8, 40)
-
-
-def _model(cfg_name, dev, train=False):
-    from prompt_tts_b200.models import TTSSingleSpeaker
-    cfg = load_cfg(cfg_name)
-    torch.manual_seed(0)
-    m = TTSSingleSpeaker(cfg).to(dev)
-    return cfg, (m if train else m.eval())
 
 
 # ---------------------------------------------------------------------------------------------------------------- loss kernel
@@ -264,20 +257,14 @@ def test_gaussian_target_kernel_loops_agree(cuda, kind, eta, n):
     """The samplers' own step code (`_step`, the fused kernels) driven by the exact predictor of x0 ~ N(0, 0.577^2), given as eps,
     x0 or v (computed in float64, rounded to fp32).  The three loops agree to 1e-5 (DESIGN section 5: an fp32 restatement of these
     steps keeps each parameterisation within 4e-7 of the float64 loop)."""
-    from prompt_tts_b200.sample import DDIMSampler, DDPMSampler, DPMSolverSampler
-    _, model = _model("tiny", cuda)
+    _, model = so.load_model("tiny", cuda)
     B, C, T, s = 25, 8, 1000, 0.577
     g = torch.Generator(device="cuda").manual_seed(5)
     x_T = torch.randn(B, C, T, device=cuda, generator=g)
     noises = torch.randn(n, B, C, T, device=cuda, generator=g)
     res = {}
     for pt in PRED:
-        if kind == "ddpm":
-            smp = DDPMSampler(model, n_infer=n, prediction_type=pt)
-        elif kind == "ddim":
-            smp = DDIMSampler(model, n_infer=n, eta=eta, prediction_type=pt)
-        else:
-            smp = DPMSolverSampler(model, n_infer=n, prediction_type=pt)
+        smp = so.make_sampler(model, kind, eta, n, pt)
         x = x_T.clone()
         smp._T = T
         smp._static = {"eps": torch.empty_like(x)}
@@ -306,26 +293,19 @@ def _oracle_train(cfg, model, inp, pt, gamma):
     return loss.detach(), {k: v.grad for k, v in sd.items() if v.requires_grad and v.grad is not None and v.grad.abs().max() > 0}
 
 
-def _grad_err(model, ref_grads):
-    named = dict(model.named_parameters())
-    keys = sorted(ref_grads)
-    assert all(named[k].grad is not None for k in keys), [k for k in keys if named[k].grad is None][:5]
-    return rel(torch.cat([named[k].grad.flatten() for k in keys]), torch.cat([ref_grads[k].flatten() for k in keys]))
-
-
 # sizes: those of test_guidance_gpu.py's condition-dropout test (test_model_gpu.py gives the reason)
 @pytest.mark.parametrize("gamma", [None, 5.0])
 @pytest.mark.parametrize("pt", NON_EPS)
 @pytest.mark.parametrize("cfg_name,B,T", [("tiny", 8, 64), ("mid", 2, 64)])
 def test_train_step_prediction_type_matches_oracle(cuda, cfg_name, B, T, pt, gamma):
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = _model(cfg_name, cuda, train=True)
+    cfg, model = so.load_model(cfg_name, cuda, train=True)
     inp = synth_inputs(cfg, B, T, seed=1, device=cuda)
     inp["t"][0] = 999
     ref_loss, ref_grads = _oracle_train(cfg, model, inp, pt, gamma)
     loss = DenoiserTrainStep(model, prediction_type=pt, snr_gamma=gamma)(inp["x0"], inp["noise"], inp["t"], inp["ids"], inp["mask"])
     torch.cuda.synchronize()
-    e_l, e_g = rel(loss, ref_loss), _grad_err(model, ref_grads)
+    e_l, e_g = rel(loss, ref_loss), so.grad_err(model, ref_grads)
     print(f"\n[{cfg_name} {B}x{T} {pt} snr_gamma={gamma}] loss {e_l:.2e} global grad {e_g:.2e}")
     assert e_l < TOL and e_g < TOL, (e_l, e_g)
 
@@ -334,7 +314,7 @@ def test_train_step_graph_replays_fresh_timesteps(cuda):
     """the Min-SNR weight and the v target are formed on the device from t: replays of one captured step with two (t, noise) pairs
     equal eager steps with the same pairs"""
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = _model("tiny", cuda, train=True)
+    cfg, model = so.load_model("tiny", cuda, train=True)
     B, T = 8, 64
     inp = synth_inputs(cfg, B, T, seed=4, device=cuda)
     stepper = DenoiserTrainStep(model, prediction_type="v_prediction", snr_gamma=5.0)
@@ -375,78 +355,16 @@ def test_train_step_graph_replays_fresh_timesteps(cuda):
 
 
 # ---------------------------------------------------------------------------------------------------------------- sampling loops
-def _sampler(model, kind, eta, n_infer, pt, use_graph=True):
-    from prompt_tts_b200.sample import DDIMSampler, DDPMSampler, DPMSolverSampler
-    if kind == "ddpm":
-        return DDPMSampler(model, n_infer=n_infer, use_graph=use_graph, prediction_type=pt)
-    if kind == "ddim":
-        return DDIMSampler(model, n_infer=n_infer, eta=eta, use_graph=use_graph, prediction_type=pt)
-    return DPMSolverSampler(model, n_infer=n_infer, use_graph=use_graph, prediction_type=pt)
-
-
-def _oracle_loop(model, cfg, kind, eta, n_infer, pt, w, ids, x_T, noises, prompt=None, prompt_noise=None, eps_err=0.0):
-    """fp32 loop: ref_model.text_encoder once, ref_model.unet (and, for w > 1, on a zero context: u + w (c - u)), the scheduler step of
-    prediction type pt; prompt frames overwritten after every step with the prompt noised to the level the step landed on.
-    eps_err > 0 adds a seeded Gaussian error of that relative size to every denoiser output."""
-    import ref_model
-    acp = ref_model.ddpm_alphas_cumprod().to(x_T.device)
-    if kind == "ddpm":
-        ts = [k * (1000 // n_infer) for k in range(n_infer)][::-1]
-    else:
-        sched = DDIMScheduler(prediction_type=pt) if kind == "ddim" else DPMSolverMultistepScheduler(prediction_type=pt)
-        sched.set_timesteps(n_infer)
-        ts = sched.timesteps.tolist()
-    sd = {k: v.detach().float() for k, v in model.state_dict().items()}
-    B = x_T.shape[0]
-    g = torch.Generator(device=x_T.device).manual_seed(29)
-
-    def err(e):
-        return e + eps_err * e.norm() / e.numel() ** 0.5 * torch.randn(e.shape, device=e.device, generator=g) if eps_err > 0 else e
-
-    with torch.no_grad():
-        enc = ref_model.text_encoder(sd, cfg, ids)
-        x = x_T.clone()
-        for i, t in enumerate(ts):
-            tt = torch.full((B,), t, device=x.device, dtype=torch.int64)
-            o = err(ref_model.unet(sd, cfg, x, tt, enc))
-            if w != 1.0:
-                u = err(ref_model.unet(sd, cfg, x, tt, torch.zeros_like(enc)))
-                o = u + w * (o - u)
-            if kind == "ddpm":
-                x = po.ddpm_step(o, t, x, noises[i], acp=acp, n_infer=n_infer, prediction_type=pt)
-                to = t - 1000 // n_infer
-            elif kind == "ddim":
-                x = sched.step(o, t, x, eta=eta, variance_noise=noises[i]).prev_sample
-                to = t - 1000 // n_infer
-            else:
-                x = sched.step(o, t, x).prev_sample
-                to = ts[i + 1] if i + 1 < n_infer else -1
-            if prompt is not None:
-                keep = prompt.shape[-1]
-                if i == n_infer - 1 or to < 0:
-                    x[..., :keep] = prompt
-                else:
-                    x[..., :keep] = acp[to].sqrt() * prompt + (1 - acp[to]).sqrt() * prompt_noise[i]
-    return x
-
-
 @pytest.fixture(scope="module")
 def tiny(cuda):
-    return _model("tiny", cuda)
-
-
-def _case(cfg, B, T, n_infer, seed, dev):
-    inp = synth_inputs(cfg, B, T, seed=seed, device=dev)
-    g = torch.Generator(device="cuda").manual_seed(seed + 100)
-    x_T = torch.randn(B, cfg["in_channels"], T, device=dev, generator=g)
-    noises = torch.randn(n_infer, B, cfg["in_channels"], T, device=dev, generator=g)
-    return inp, x_T, noises
+    return so.load_model("tiny", cuda)
 
 
 def _bound(model, cfg, kind, eta, n_infer, pt, w, inp, x_T, noises, want, prompt=None, pn=None):
     """what the fp32 oracle loop makes of the 2e-2 per-call bar (DESIGN section 5), and at least that bar doubled (the bound of the
     stochastic loops in test_fast_sampler_gpu.py)"""
-    e = rel(_oracle_loop(model, cfg, kind, eta, n_infer, pt, w, inp["ids"], x_T, noises, prompt, pn, eps_err=TOL), want)
+    e = rel(so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, pt=pt, w=w, prompt=prompt, prompt_noise=pn,
+                           eps_err=TOL, err_seed=29), want)
     return max(e, 2 * TOL)
 
 
@@ -458,13 +376,14 @@ KINDS = [("ddpm", None), ("ddim", 0.0), ("ddim", 1.0), ("dpm", None)]
 def test_sampler_loop_matches_oracle(cuda, tiny, kind, eta, pt):
     cfg, model = tiny
     B, T, n_infer = 2, 16, 5
-    inp, x_T, noises = _case(cfg, B, T, n_infer, 5, cuda)
-    outs = {gr: _sampler(model, kind, eta, n_infer, pt, gr).sample(inp["ids"], T, x_T=x_T, noises=noises) for gr in (False, True)}
+    inp, x_T, noises = so.case(cfg, B, T, n_infer, 5, cuda)
+    outs = {gr: so.make_sampler(model, kind, eta, n_infer, pt, gr).sample(inp["ids"], T, x_T=x_T, noises=noises)
+            for gr in (False, True)}
     # GroupNorm statistics are accumulated with fp32 atomics (order not fixed), so two runs agree to rounding, not bit for bit
     assert rel(outs[False], outs[True]) < 1e-3, "graph replay must reproduce the eager loop"
-    want = _oracle_loop(model, cfg, kind, eta, n_infer, pt, 1.0, inp["ids"], x_T, noises)
-    eps_loop = _oracle_loop(model, cfg, kind, eta, n_infer, "epsilon", 1.0, inp["ids"], x_T, noises)
-    bound = _bound(model, cfg, kind, eta, n_infer, pt, 1.0, inp, x_T, noises, want)
+    want = so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, pt=pt)
+    eps_loop = so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises)
+    bound = _bound(model, cfg, kind, eta, n_infer, pt, None, inp, x_T, noises, want)
     e = {gr: rel(outs[gr], want) for gr in (False, True)}
     print(f"\n[{kind} eta={eta} {pt} tiny, {n_infer} steps] rel err vs fp32 oracle loop: graph {e[True]:.2e}, eager {e[False]:.2e} "
           f"(bound {bound:.2e}; vs the epsilon reading of the same model {rel(want, eps_loop):.2e})")
@@ -475,9 +394,9 @@ def test_sampler_loop_matches_oracle(cuda, tiny, kind, eta, pt):
 def test_guided_sampler_loop_matches_oracle(cuda, tiny, pt):
     cfg, model = tiny
     B, T, n_infer, w = 2, 16, 5, 3.0
-    inp, x_T, noises = _case(cfg, B, T, n_infer, 6, cuda)
-    got = _sampler(model, "ddim", 0.0, n_infer, pt).sample(inp["ids"], T, x_T=x_T, noises=noises, guidance_scale=w)
-    want = _oracle_loop(model, cfg, "ddim", 0.0, n_infer, pt, w, inp["ids"], x_T, noises)
+    inp, x_T, noises = so.case(cfg, B, T, n_infer, 6, cuda)
+    got = so.make_sampler(model, "ddim", 0.0, n_infer, pt).sample(inp["ids"], T, x_T=x_T, noises=noises, guidance_scale=w)
+    want = so.oracle_loop(model, cfg, "ddim", 0.0, n_infer, inp["ids"], x_T, noises, pt=pt, w=w)
     bound = _bound(model, cfg, "ddim", 0.0, n_infer, pt, w, inp, x_T, noises, want)
     print(f"\n[guided ddim {pt} w={w}] rel err {rel(got, want):.2e} (bound {bound:.2e})")
     assert rel(got, want) < bound
@@ -488,13 +407,13 @@ def test_guided_sampler_loop_matches_oracle(cuda, tiny, pt):
 def test_sampler_prompt_inpainting_matches_oracle(cuda, tiny, kind, eta, pt):
     cfg, model = tiny
     B, T, P, n_infer = 2, 16, 6, 4
-    inp, x_T, noises = _case(cfg, B, T, n_infer, 7, cuda)
+    inp, x_T, noises = so.case(cfg, B, T, n_infer, 7, cuda)
     prompt = inp["x0"][..., :P].contiguous()
     g = torch.Generator(device="cuda").manual_seed(13)
     pn = torch.randn(n_infer, B, cfg["in_channels"], P, device=cuda, generator=g)
-    got = _sampler(model, kind, eta, n_infer, pt).sample(inp["ids"], T, x_T=x_T, noises=noises, prompt=prompt, prompt_noise=pn)
-    want = _oracle_loop(model, cfg, kind, eta, n_infer, pt, 1.0, inp["ids"], x_T, noises, prompt, pn)
-    bound = _bound(model, cfg, kind, eta, n_infer, pt, 1.0, inp, x_T, noises, want, prompt, pn)
+    got = so.make_sampler(model, kind, eta, n_infer, pt).sample(inp["ids"], T, x_T=x_T, noises=noises, prompt=prompt, prompt_noise=pn)
+    want = so.oracle_loop(model, cfg, kind, eta, n_infer, inp["ids"], x_T, noises, pt=pt, prompt=prompt, prompt_noise=pn)
+    bound = _bound(model, cfg, kind, eta, n_infer, pt, None, inp, x_T, noises, want, prompt, pn)
     print(f"\n[{kind} {pt} + prompt] rel err {rel(got, want):.2e} (bound {bound:.2e})")
     assert torch.equal(got[..., :P], prompt), "the prompt frames must come out clean"
     assert rel(got, want) < bound
@@ -523,9 +442,9 @@ def _count(fn, monkeypatch):
 
 def test_launch_counts(cuda, monkeypatch):
     """The default train step still launches add_noise + mse_fwd_bwd, a non-default one add_noise + diffusion_loss: the same count.
-    The default samplers call the entry points without the suffix, the others the `_pred` variants: the same count."""
+    Every sampler calls its `_pred` step entry point once per step whatever the type, and launches as many kernels for each type."""
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = _model("tiny", cuda, train=True)
+    cfg, model = so.load_model("tiny", cuda, train=True)
     B, T = 8, 64
     inp = synth_inputs(cfg, B, T, seed=9, device=cuda)
     counts = {}
@@ -543,10 +462,10 @@ def test_launch_counts(cuda, monkeypatch):
     for kind, eta, step in (("ddpm", None, "ddpm_step"), ("ddim", 1.0, "ddim_step"), ("dpm", None, "dpmpp_step")):
         c = {}
         for pt in PRED:
-            smp = _sampler(model, kind, eta, n_infer, pt)
+            smp = so.make_sampler(model, kind, eta, n_infer, pt)
             smp.sample(inp["ids"], T, seed=1)
             n, names = _count(lambda: smp.sample(inp["ids"], T, seed=1), monkeypatch)
-            want = step if pt == "epsilon" else step + "_pred"
+            want = step + "_pred"
             assert names.count(want) == n_infer and not any(s.startswith(step) and s != want for s in names), (kind, pt, names)
             c[pt] = n
         assert len(set(c.values())) == 1, (kind, c)

@@ -3,7 +3,8 @@ diffusers 0.15 `DDPMScheduler.step` / the reference denoiser (oracle/ref_model.p
 import pytest
 import torch
 
-from util import load_cfg, rel, synth_inputs
+import sampling_oracle as so
+from util import rel, synth_inputs
 
 pytestmark = pytest.mark.gpu
 
@@ -26,12 +27,8 @@ def test_ddpm_step_matches_oracle(cuda, t):
 
 
 def test_sampler_matches_oracle_loop(cuda):
-    import ref_model
-    from prompt_tts_b200.models import TTSSingleSpeaker
     from prompt_tts_b200.sample import DDPMSampler
-    cfg = load_cfg("tiny")
-    torch.manual_seed(0)
-    model = TTSSingleSpeaker(cfg).to(cuda).eval()
+    cfg, model = so.load_model("tiny", cuda)
     B, T, n_infer = 2, 16, 5
     inp = synth_inputs(cfg, B, T, seed=5, device=cuda)
     g = torch.Generator(device="cuda").manual_seed(9)
@@ -43,25 +40,15 @@ def test_sampler_matches_oracle_loop(cuda):
     # GroupNorm statistics are accumulated with fp32 atomics (order not fixed), so two runs agree to rounding, not bit for bit
     assert rel(outs[False], outs[True]) < 1e-3, "graph replay must reproduce the eager loop"
     # oracle loop: fp32 reference modules + DDPMScheduler.step restatement, same x_T / noises
-    sd = {k: v.detach().float() for k, v in model.state_dict().items()}
-    with torch.no_grad():
-        enc = ref_model.text_encoder(sd, cfg, inp["ids"])
-        x = x_T.clone()
-        stride = 1000 // n_infer
-        for i, t in enumerate([k * stride for k in range(n_infer)][::-1]):
-            eps = ref_model.unet(sd, cfg, x, torch.full((B,), t, device=cuda, dtype=torch.int64), enc)
-            x = ref_model.ddpm_step(eps, t, x, noises[i], acp=ref_model.ddpm_alphas_cumprod().to(cuda), n_infer=n_infer)
+    x = so.oracle_loop(model, cfg, "ddpm", None, n_infer, inp["ids"], x_T, noises)
     e = rel(outs[True], x)
     print(f"\n[sampler tiny, {n_infer} steps] rel err vs fp32 oracle loop {e:.2e}")
     assert e < 2e-2 * 2, e          # bf16 denoiser error (<= 2e-2 per call) compounds over the steps; the scheduler step itself is exact
 
 
 def test_sampler_prompt_inpainting_and_codes(cuda):
-    from prompt_tts_b200.models import TTSSingleSpeaker
     from prompt_tts_b200.sample import DDPMSampler
-    cfg = load_cfg("tiny")
-    torch.manual_seed(0)
-    model = TTSSingleSpeaker(cfg).to(cuda).eval()
+    cfg, model = so.load_model("tiny", cuda)
     B, T, P = 2, 16, 6
     inp = synth_inputs(cfg, B, T, seed=6, device=cuda)
     prompt = inp["x0"][..., :P].contiguous()
@@ -78,12 +65,8 @@ def test_sampler_prompt_inpainting_and_codes(cuda):
 def test_sampler_prompt_tokens_extend_the_cross_attention_context(cuda):
     """Optional speech-prompt tokens appended to the text encoding (SURVEY 8 row N2 hook, default off): the run with tokens equals
     the oracle loop whose encoder_hidden_states is [text encoding | tokens], and differs from the run without them."""
-    import ref_model
-    from prompt_tts_b200.models import TTSSingleSpeaker
     from prompt_tts_b200.sample import DDPMSampler
-    cfg = load_cfg("tiny")
-    torch.manual_seed(0)
-    model = TTSSingleSpeaker(cfg).to(cuda).eval()
+    cfg, model = so.load_model("tiny", cuda)
     B, T, n_infer, P = 2, 16, 3, 9
     inp = synth_inputs(cfg, B, T, seed=8, device=cuda)
     g = torch.Generator(device="cuda").manual_seed(4)
@@ -94,12 +77,5 @@ def test_sampler_prompt_tokens_extend_the_cross_attention_context(cuda):
     with_t = smp.sample(inp["ids"], T, x_T=x_T, noises=noises, prompt_tokens=toks)
     without = smp.sample(inp["ids"], T, x_T=x_T, noises=noises)
     assert rel(with_t, without) > 1e-3
-    sd = {k: v.detach().float() for k, v in model.state_dict().items()}
-    with torch.no_grad():
-        enc = torch.cat([ref_model.text_encoder(sd, cfg, inp["ids"]), toks], dim=1)
-        x = x_T.clone()
-        stride = 1000 // n_infer
-        for i, t in enumerate([k * stride for k in range(n_infer)][::-1]):
-            eps = ref_model.unet(sd, cfg, x, torch.full((B,), t, device=cuda, dtype=torch.int64), enc)
-            x = ref_model.ddpm_step(eps, t, x, noises[i], acp=ref_model.ddpm_alphas_cumprod().to(cuda), n_infer=n_infer)
+    x = so.oracle_loop(model, cfg, "ddpm", None, n_infer, inp["ids"], x_T, noises, toks=toks)
     assert rel(with_t, x) < 4e-2

@@ -119,6 +119,16 @@ def test_fast_samplers_check_their_arguments(cpu_model):
             smp.sample(torch.zeros(1, 24, dtype=torch.int32), 16)
 
 
+def test_ddpm_sampler_checks_n_infer(cpu_model):
+    """n_infer = 0 would divide by zero and n_infer > n_train would give a zero stride (every timestep 0)"""
+    from prompt_tts_b200.sample import DDPMSampler
+    for bad, n_train in ((0, 1000), (1001, 1000), (11, 10), (True, 1000), (2.5, 1000), ("5", 1000)):
+        with pytest.raises(ValueError, match="n_infer"):
+            DDPMSampler(cpu_model, n_infer=bad, n_train=n_train)
+    assert DDPMSampler(cpu_model).n_infer == 100 and DDPMSampler(cpu_model, n_infer=10, n_train=10).stride == 1
+    assert DDPMSampler(cpu_model, n_infer=5.0).timesteps == [800, 600, 400, 200, 0]
+
+
 def test_step_entry_points_validate_their_scalars():
     """pt_ddim_step / pt_dpmpp_step refuse bad scalars before anything is launched (no device needed).  Pointers are never
     dereferenced on these paths: each call fails validation first."""
