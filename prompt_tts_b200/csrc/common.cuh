@@ -70,6 +70,16 @@ static inline int pt_num_sms() {
   return n > 1 ? n : 1;
 }
 
+// Grid of a grid-stride kernel: one block per `per_block` items, at most `waves` blocks per SM
+static inline unsigned grid_for(long long items, int per_block, int waves = 8) {
+  long long b = (items + per_block - 1) / per_block;
+  const long long cap = (long long)pt_num_sms() * waves;
+  if (b > cap) b = cap;
+  if (b < 1) b = 1;
+  return (unsigned)b;
+}
+static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -78,6 +88,19 @@ __device__ __forceinline__ float warp_sum(float v) {
 __device__ __forceinline__ float warp_max(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
+  return v;
+}
+// Sum of `acc` over the block (blockDim.x a multiple of 32), valid in thread 0.  Call it from every thread: it synchronises.
+__device__ __forceinline__ float block_sum(float acc) {
+  acc = warp_sum(acc);
+  __shared__ float sh[32];
+  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  float v = 0.f;
+  if (threadIdx.x < 32) {
+    v = threadIdx.x < (blockDim.x >> 5) ? sh[threadIdx.x] : 0.f;
+    v = warp_sum(v);
+  }
   return v;
 }
 

@@ -27,12 +27,12 @@ import torch
 
 from . import engine as E
 from . import ops
+from .sample import ddpm_alphas_cumprod
 
 
 def ddpm_tables(n: int = 1000, beta_start: float = 1e-4, beta_end: float = 0.02, device="cuda"):
     """sqrt(alphas_cumprod), sqrt(1 - alphas_cumprod) of the linear-beta DDPM schedule (train.py:32-36)."""
-    betas = torch.linspace(beta_start, beta_end, n, dtype=torch.float32)
-    acp = torch.cumprod(1.0 - betas, 0)
+    acp = ddpm_alphas_cumprod(n, beta_start, beta_end)
     return (acp ** 0.5).to(device), ((1 - acp) ** 0.5).to(device)
 
 
