@@ -173,10 +173,16 @@ def velocity(x0, noise, t):
     return DDPMScheduler(prediction_type="v_prediction").get_velocity(x0, noise, t)
 
 
-def train_step_loss(sd, cfg, codes, noise, t, ids, mask=None, prediction_type="epsilon", snr_gamma=None):
+def train_step_loss(sd, cfg, codes, noise, t, ids, mask=None, prediction_type="epsilon", snr_gamma=None, cond_keep=None):
     """ref_model.train_step_loss with the target of `prediction_type` (noise, x0 or the velocity) and, for snr_gamma not None,
-    the training examples' Min-SNR-gamma weighting: mean over samples of w_b * the sample's MSE."""
-    pred = ref_model.tts_forward(sd, cfg, ref_model.add_noise(codes, noise, t), t, ids, mask)
+    the training examples' Min-SNR-gamma weighting: mean over samples of w_b * the sample's MSE.  cond_keep (bool [B]): condition
+    dropout, the text encoding of every dropped row replaced by zeros."""
+    xt = ref_model.add_noise(codes, noise, t)
+    if cond_keep is None:
+        pred = ref_model.tts_forward(sd, cfg, xt, t, ids, mask)
+    else:
+        enc = ref_model.text_encoder(sd, cfg, ids)
+        pred = ref_model.unet(sd, cfg, xt, t, torch.where(cond_keep[:, None, None], enc, 0))
     target = {"epsilon": noise, "sample": codes}.get(prediction_type)
     if target is None:
         assert prediction_type == "v_prediction", prediction_type

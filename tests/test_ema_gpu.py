@@ -5,22 +5,20 @@ the launch count and two data-parallel ranks.
 Two forward/backward passes of the train step are not bit-identical (GroupNorm statistics and weight gradients are accumulated with
 fp32 atomics), so where two runs are compared bit for bit the second one is fed the gradients the first one computed: what is
 compared is the optimiser and the EMA, which are deterministic."""
-import json
 import math
 import os
-import subprocess
 import sys
 
 import pytest
 import torch
 
-from util import ROOT, load_cfg, rel, synth_inputs
+import training_oracle as to
+from util import ROOT, load_model, rel
 
 sys.path.insert(0, os.path.join(ROOT, "oracle", "diffusers_shim"))
 from diffusers.training_utils import EMAModel  # noqa: E402
 
 pytestmark = pytest.mark.gpu
-KW = dict(lr=1e-3, betas=(0.95, 0.999), weight_decay=1e-2, eps=1e-8, max_norm=0.05)     # a few steps move the weights measurably
 # warmup: the device's double pow() and the host's may differ in the last bits of 1 - (1 + step / inv_gamma) ** -power (CUDA
 # documents pow to 2 ulp, glibc to 1).  Near decay ~ 1 that is a few ulp of 1.0 in the decay, and at most one fp32 ulp in the
 # coefficient 1 - decay when it falls on a rounding boundary; over a few steps the average then differs by far less than this.
@@ -28,20 +26,6 @@ WARMUP_DECAY_ATOL = 2.0 ** -50
 WARMUP_EMA_REL = 1e-6
 VARIANTS = {"default": {}, "update_after_step=2": dict(update_after_step=2), "min_decay=0.5": dict(decay=0.9, min_decay=0.5),
             "warmup": dict(use_ema_warmup=True, inv_gamma=1.0, power=2 / 3)}
-
-
-def _setup(cuda, cfg_name="tiny", B=2, T=16, seed=2, accumulation_steps=1, ema_kw=None, model_seed=0):
-    from prompt_tts_b200.models import TTSSingleSpeaker
-    from prompt_tts_b200.optim import FusedClipAdamW, FusedEMA
-    from prompt_tts_b200.train import DenoiserTrainStep
-    cfg = load_cfg(cfg_name)
-    torch.manual_seed(model_seed)
-    model = TTSSingleSpeaker(cfg).to(cuda)
-    inp = synth_inputs(cfg, B, T, seed=seed, device=cuda)
-    stepper = DenoiserTrainStep(model, accumulation_steps=accumulation_steps)
-    opt = FusedClipAdamW(stepper, **KW)
-    ema = FusedEMA(opt, **(ema_kw or {})) if ema_kw is not None else None
-    return cfg, model, inp, stepper, opt, ema
 
 
 def _run(stepper, inp, sl=slice(None)):
@@ -135,7 +119,7 @@ def test_device_decay_schedule_matches_shim(cuda, kw):
 def test_ema_matches_shim_end_to_end(cuda, cfg_name, variant):
     from prompt_tts_b200.models import TTSSingleSpeaker
     kw = VARIANTS[variant]
-    cfg, model, inp, stepper, opt, ema = _setup(cuda, cfg_name, ema_kw=kw)
+    cfg, model, inp, stepper, opt, ema = to.setup(cuda, cfg_name, ema_kw=kw)
     shim = EMAModel(model.parameters(), **kw)
     for _ in range(5):
         _run(stepper, inp)
@@ -155,7 +139,7 @@ def test_ema_matches_shim_end_to_end(cuda, cfg_name, variant):
 
 def test_ema_constructed_after_attach_starts_from_current_weights(cuda):
     from prompt_tts_b200.optim import FusedEMA
-    cfg, model, inp, stepper, opt, _ = _setup(cuda)
+    cfg, model, inp, stepper, opt, _ = to.setup(cuda)
     for _ in range(2):
         _run(stepper, inp)
         opt.step()
@@ -169,23 +153,10 @@ def test_ema_constructed_after_attach_starts_from_current_weights(cuda):
 
 
 # ------------------------------------------------------------------------------------------------ 4. graph capture
-def _capture(fn):
-    side = torch.cuda.Stream()                                                # warm-up on a side stream, as torch asks before capture
-    side.wait_stream(torch.cuda.current_stream())
-    with torch.cuda.stream(side):
-        fn()
-    torch.cuda.current_stream().wait_stream(side)
-    torch.cuda.synchronize()
-    g = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(g):
-        fn()
-    return g
-
-
 def test_ema_graph_replays(cuda):
     """One captured `step(); opt.step()` replayed: the EMA's step counter and decay live in device memory, so every replay is the
     next EMA step."""
-    cfg, model, inp, stepper, opt, ema = _setup(cuda, ema_kw={})
+    cfg, model, inp, stepper, opt, ema = to.setup(cuda, ema_kw={})
     shim = EMAModel(model.parameters())
 
     def full():
@@ -194,7 +165,7 @@ def test_ema_graph_replays(cuda):
 
     full()                                  # eager step 1 (defines the flat layout, starts the average)
     shim.step(model.parameters())
-    g = _capture(full)                      # eager step 2 on the side stream, then the capture (which runs nothing)
+    g = to.capture(full)                    # eager step 2 on the side stream, then the capture (which runs nothing)
     shim.step(model.parameters())
     _check_against_shim(model, ema, shim)
     for _ in range(5):
@@ -206,7 +177,7 @@ def test_ema_graph_replays(cuda):
 
 
 def test_ema_steps_once_per_accumulation_window_in_a_graph(cuda):
-    cfg, model, inp, stepper, opt, ema = _setup(cuda, B=4, accumulation_steps=2, ema_kw=dict(decay=0.9))
+    cfg, model, inp, stepper, opt, ema = to.setup(cuda, B=4, accumulation_steps=2, ema_kw=dict(decay=0.9))
     shim = EMAModel(model.parameters(), decay=0.9)
 
     def window():
@@ -216,7 +187,7 @@ def test_ema_steps_once_per_accumulation_window_in_a_graph(cuda):
 
     window()
     shim.step(model.parameters())
-    g = _capture(window)
+    g = to.capture(window)
     shim.step(model.parameters())           # the warm-up window
     _check_against_shim(model, ema, shim)
     for _ in range(3):
@@ -230,9 +201,8 @@ def test_ema_steps_once_per_accumulation_window_in_a_graph(cuda):
 # ------------------------------------------------------------------------------------------------ 5. swapped()
 def test_swapped_samples_the_ema_and_restores_everything(cuda):
     from prompt_tts_b200 import _lib
-    from prompt_tts_b200.models import TTSSingleSpeaker
     from prompt_tts_b200.sample import DDIMSampler
-    cfg, model, inp, stepper, opt, ema = _setup(cuda, ema_kw=dict(decay=0.9))
+    cfg, model, inp, stepper, opt, ema = to.setup(cuda, ema_kw=dict(decay=0.9))
     for _ in range(3):
         _run(stepper, inp)
         opt.step()
@@ -243,7 +213,7 @@ def test_swapped_samples_the_ema_and_restores_everything(cuda):
         stepper.grad_sync.flat.copy_(gfix)
         opt.step()
 
-    g = _capture(train)                             # a training graph captured before the swap
+    g = to.capture(train)                           # a training graph captured before the swap
     torch.cuda.synchronize()
     bufs = lambda: [opt.pflat, opt.wflat, opt.m, opt.v, ema.eflat, opt.state, ema.state]     # noqa: E731
     before = [b.clone() for b in bufs()]
@@ -261,8 +231,7 @@ def test_swapped_samples_the_ema_and_restores_everything(cuda):
         got = DDIMSampler(model, n_infer=3).sample(inp["ids"], 16, x_T=x_T)
     for b, w in zip(bufs(), before):
         assert torch.equal(b, w)
-    torch.manual_seed(9)
-    fresh = TTSSingleSpeaker(cfg).to(cuda)
+    _, fresh = load_model("tiny", cuda, train=True, seed=9)
     fresh.load_state_dict(ema_sd, strict=True)
     want = DDIMSampler(fresh, n_infer=3).sample(inp["ids"], 16, x_T=x_T)
     assert torch.equal(got, want), rel(got, want)
@@ -282,7 +251,7 @@ def test_swapped_samples_the_ema_and_restores_everything(cuda):
 
 def test_swapped_refuses_capture_and_copy_to_is_permanent(cuda):
     from prompt_tts_b200 import _lib
-    cfg, model, inp, stepper, opt, ema = _setup(cuda, ema_kw=dict(decay=0.9))
+    cfg, model, inp, stepper, opt, ema = to.setup(cuda, ema_kw=dict(decay=0.9))
     for _ in range(2):
         _run(stepper, inp)
         opt.step()
@@ -302,11 +271,10 @@ def test_swapped_refuses_capture_and_copy_to_is_permanent(cuda):
 # ------------------------------------------------------------------------------------------------ 6. resume
 def test_resume_is_bit_identical(cuda):
     from prompt_tts_b200 import _lib
-    from prompt_tts_b200.models import TTSSingleSpeaker
     from prompt_tts_b200.optim import FusedClipAdamW, FusedEMA
     from prompt_tts_b200.train import DenoiserTrainStep
     ema_kw = dict(decay=0.95, update_after_step=1, min_decay=0.1)
-    cfg, model, inp, stepper, opt, ema = _setup(cuda, ema_kw=ema_kw)
+    cfg, model, inp, stepper, opt, ema = to.setup(cuda, ema_kw=ema_kw)
     for _ in range(3):
         _run(stepper, inp)
         opt.step()
@@ -318,11 +286,10 @@ def test_resume_is_bit_identical(cuda):
         opt.step()
     torch.cuda.synchronize()
     # resume into fresh objects (other initial weights, default EMA hyper-parameters: the checkpoint's are restored)
-    torch.manual_seed(5)
-    model2 = TTSSingleSpeaker(cfg).to(cuda)
+    _, model2 = load_model("tiny", cuda, train=True, seed=5)
     model2.load_state_dict(ck[0], strict=True)
     stepper2 = DenoiserTrainStep(model2)
-    opt2 = FusedClipAdamW(stepper2, **KW)
+    opt2 = FusedClipAdamW(stepper2, **to.OPT_KW)
     ema2 = FusedEMA(opt2)
     for k in range(2):
         _run(stepper2, inp)
@@ -348,7 +315,7 @@ def test_opt_step_launch_count(cuda):
     lib = _lib.lib()
     counts = {}
     for with_ema in (False, True):
-        cfg, model, inp, stepper, opt, ema = _setup(cuda, ema_kw={} if with_ema else None)
+        cfg, model, inp, stepper, opt, ema = to.setup(cuda, ema_kw={} if with_ema else None)
         _run(stepper, inp)
         opt.step()                              # attach (one cast of the shadow) happens here
         _run(stepper, inp)
@@ -360,15 +327,7 @@ def test_opt_step_launch_count(cuda):
 
 # ------------------------------------------------------------------------------------------------ 8. two ranks
 def test_two_rank_ema_identical(cuda):
-    n = torch.cuda.device_count()
-    if n < 2:
-        pytest.skip("needs two GPUs")
-    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
-           "--master-port", "29543", os.path.join(ROOT, "tests", "ema_dp_worker.py"), "tiny3", "2", "64"]
-    r = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)
-    assert r.returncode == 0, (r.stdout[-1500:], r.stderr[-3000:])
-    res = json.loads([l for l in r.stdout.splitlines() if l.startswith("EMARESULT ")][-1][len("EMARESULT "):])
-    print(res)
+    res = to.run_two_ranks("ema", "tiny3", 2, 64, 29543)
     for mode in ("fp32", "bf16"):
         assert res[mode]["optimization_step"] == 3
         assert res[mode]["ema_identical_on_all_ranks"] and res[mode]["weights_identical_on_all_ranks"], res

@@ -8,7 +8,7 @@ import pytest
 import torch
 
 import sampling_oracle as so
-from util import ROOT, rel, synth_inputs
+from util import ROOT, load_model, rel, synth_inputs
 
 sys.path.insert(0, os.path.join(ROOT, "oracle", "diffusers_shim"))
 from diffusers.schedulers_few_step import DDIMScheduler, DPMSolverMultistepScheduler  # noqa: E402
@@ -110,7 +110,7 @@ SAMPLERS = [("ddim", 0.0), ("ddim", 1.0), ("dpm", None)]
 
 @pytest.fixture(scope="module")
 def tiny(cuda):
-    return so.load_model("tiny", cuda)
+    return load_model("tiny", cuda)
 
 
 @pytest.mark.parametrize("kind,eta", SAMPLERS)

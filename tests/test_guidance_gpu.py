@@ -7,7 +7,8 @@ import pytest
 import torch
 
 import sampling_oracle as so
-from util import rel, synth_inputs
+import training_oracle as to
+from util import load_model, rel, synth_inputs
 
 pytestmark = pytest.mark.gpu
 TOL = 2e-2
@@ -111,7 +112,7 @@ def test_block_null_context_shortcut_is_exact(cuda, dim, ctx, Lk, B):
 def test_guided_forward_matches_oracle(cuda, cfg_name):
     import ref_model
     from prompt_tts_b200 import engine as E
-    cfg, model = so.load_model(cfg_name, cuda)
+    cfg, model = load_model(cfg_name, cuda)
     B, T = 1, 752
     inp = synth_inputs(cfg, B, T, seed=4, device=cuda)
     x = inp["noise"]
@@ -138,7 +139,7 @@ KINDS = [("ddpm", None), ("ddim", 0.0), ("ddim", 1.0), ("dpm", None)]
 
 @pytest.fixture(scope="module")
 def tiny(cuda):
-    return so.load_model("tiny", cuda)
+    return load_model("tiny", cuda)
 
 
 @pytest.mark.parametrize("kind,eta", KINDS)
@@ -232,19 +233,6 @@ def test_guidance_one_is_the_unguided_loop(cuda, tiny):
 
 
 # ---------------------------------------------------------------------------------------------------------------- training
-def _oracle_train(cfg, model, inp, keep):
-    """add_noise, the text encoding selected by keep (zeros where dropped), the UNet, MSE: fp32 autograd"""
-    import ref_model
-    sd = {k: v.detach().clone().requires_grad_(v.is_floating_point() and "inv_freq" not in k) for k, v in model.state_dict().items()}
-    xt = ref_model.add_noise(inp["x0"], inp["noise"], inp["t"])
-    enc = ref_model.text_encoder(sd, cfg, inp["ids"])
-    enc = torch.where(keep.bool()[:, None, None], enc, torch.zeros_like(enc))
-    pred = ref_model.unet(sd, cfg, xt, inp["t"], enc)
-    loss = torch.nn.functional.mse_loss(pred, inp["noise"])
-    loss.backward()
-    return xt, loss.detach(), {k: v.grad for k, v in sd.items() if v.requires_grad and v.grad is not None and v.grad.abs().max() > 0}
-
-
 def _keep(B, dev):
     return (torch.arange(B, device=dev) % 3 != 1)          # mixed: 1, 0, 1, 1, 0, 1, ...
 
@@ -253,11 +241,11 @@ def _keep(B, dev):
 @pytest.mark.parametrize("cfg_name,B,T", [("tiny", 8, 64), ("tiny3", 8, 128), ("mid", 2, 64)])
 def test_train_step_condition_dropout_matches_oracle(cuda, cfg_name, B, T):
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = so.load_model(cfg_name, cuda, train=True)
+    cfg, model = load_model(cfg_name, cuda, train=True)
     inp = synth_inputs(cfg, B, T, seed=1, device=cuda)
     keep = _keep(B, cuda)
     assert keep.any() and not keep.all()
-    _, ref_loss, ref_grads = _oracle_train(cfg, model, inp, keep)
+    _, _, ref_loss, ref_grads = to.oracle_train(cfg, model, inp, cond_keep=keep)
     loss = DenoiserTrainStep(model)(inp["x0"], inp["noise"], inp["t"], inp["ids"], inp["mask"], cond_keep=keep)
     torch.cuda.synchronize()
     e_l, e_g = rel(loss, ref_loss), so.grad_err(model, ref_grads)
@@ -267,7 +255,7 @@ def test_train_step_condition_dropout_matches_oracle(cuda, cfg_name, B, T):
 
 def test_train_step_all_dropped(cuda):
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = so.load_model("tiny", cuda, train=True)
+    cfg, model = load_model("tiny", cuda, train=True)
     B, T = 8, 64
     inp = synth_inputs(cfg, B, T, seed=2, device=cuda)
     none = torch.zeros(B, dtype=torch.bool, device=cuda)
@@ -292,63 +280,38 @@ def test_train_step_all_dropped(cuda):
 
 def test_train_step_all_kept_is_the_default(cuda):
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = so.load_model("tiny", cuda, train=True)
+    cfg, model = load_model("tiny", cuda, train=True)
     B, T = 8, 64
     inp = synth_inputs(cfg, B, T, seed=3, device=cuda)
     stepper = DenoiserTrainStep(model)
-    named = list(model.named_parameters())
     l_none = float(stepper(inp["x0"], inp["noise"], inp["t"], inp["ids"]))
-    g_none = torch.cat([p.grad.flatten() for _, p in named if p.grad is not None]).clone()
+    g_none = to.flat_grads(model)
     l_all = float(stepper(inp["x0"], inp["noise"], inp["t"], inp["ids"], cond_keep=torch.ones(B, dtype=torch.uint8, device=cuda)))
-    g_all = torch.cat([p.grad.flatten() for _, p in named if p.grad is not None])
+    g_all = to.flat_grads(model)
     assert abs(l_none - l_all) <= 1e-3 * abs(l_none) and rel(g_all, g_none) < 1e-3
 
 
 def test_train_step_graph_replays_fresh_masks(cuda):
     """a captured step reads the mask from its static buffer: replays with two masks equal eager steps with the same masks"""
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = so.load_model("tiny", cuda, train=True)
+    cfg, model = load_model("tiny", cuda, train=True)
     B, T = 8, 64
     inp = synth_inputs(cfg, B, T, seed=4, device=cuda)
     stepper = DenoiserTrainStep(model)
     keep = torch.ones(B, dtype=torch.bool, device=cuda)
-    loss = torch.zeros((), device=cuda)
     masks = [_keep(B, cuda), torch.arange(B, device=cuda) % 2 == 0]
-    named = list(model.named_parameters())
-
-    def step():
-        return stepper(inp["x0"], inp["noise"], inp["t"], inp["ids"], loss_out=loss, cond_keep=keep)
-
-    eager = []
-    for m in masks:
-        keep.copy_(m)
-        step()
-        torch.cuda.synchronize()
-        eager.append((float(loss), torch.cat([p.grad.flatten() for _, p in named if p.grad is not None]).clone()))
-    side = torch.cuda.Stream()
-    side.wait_stream(torch.cuda.current_stream())
-    with torch.cuda.stream(side):
-        step()
-    torch.cuda.current_stream().wait_stream(side)
-    torch.cuda.synchronize()
-    graph = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(graph):
-        step()
-    for m, (l_e, g_e) in zip(masks, eager):
-        keep.copy_(m)
-        graph.replay()
-        torch.cuda.synchronize()
-        g = torch.cat([p.grad.flatten() for _, p in named if p.grad is not None])
-        assert abs(float(loss) - l_e) <= 1e-3 * abs(l_e) and rel(g, g_e) < 1e-3
+    eager = to.check_replays_fresh_inputs(
+        model, lambda loss: stepper(inp["x0"], inp["noise"], inp["t"], inp["ids"], loss_out=loss, cond_keep=keep), [keep],
+        [[m] for m in masks])
     assert rel(eager[0][1], eager[1][1]) > 1e-3, "the two masks must give different gradients"
 
 
 def test_model_forward_cond_keep_matches_oracle(cuda):
-    cfg, model = so.load_model("tiny", cuda, train=True)
+    cfg, model = load_model("tiny", cuda, train=True)
     B, T = 8, 64
     inp = synth_inputs(cfg, B, T, seed=5, device=cuda)
     keep = _keep(B, cuda)
-    xt, ref_loss, ref_grads = _oracle_train(cfg, model, inp, keep)
+    xt, _, ref_loss, ref_grads = to.oracle_train(cfg, model, inp, cond_keep=keep)
     out = model(xt, inp["t"], inp["ids"], inp["mask"], cond_keep=keep).sample
     loss = torch.nn.functional.mse_loss(out, inp["noise"])
     loss.backward()
@@ -361,7 +324,7 @@ def test_model_forward_cond_keep_matches_oracle(cuda):
 def test_bad_cond_keep_raises(cuda):
     from prompt_tts_b200 import _lib
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = so.load_model("tiny", cuda, train=True)
+    cfg, model = load_model("tiny", cuda, train=True)
     B, T = 2, 16
     inp = synth_inputs(cfg, B, T, seed=6, device=cuda)
     stepper = DenoiserTrainStep(model)

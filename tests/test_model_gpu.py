@@ -3,30 +3,11 @@ inputs and an identical state_dict.  Tolerance: north-star 2e-2 relative (bf16 c
 import pytest
 import torch
 
-from util import load_cfg, rel, synth_inputs
+import training_oracle as to
+from util import load_model, rel, synth_inputs
 
 pytestmark = pytest.mark.gpu
 TOL = 2e-2
-
-
-def _oracle(cfg, sd, inp):
-    import ref_model
-    sd = {k: v.detach().clone().requires_grad_(v.is_floating_point() and "inv_freq" not in k) for k, v in sd.items()}
-    xt = ref_model.add_noise(inp["x0"], inp["noise"], inp["t"])
-    pred = ref_model.tts_forward(sd, cfg, xt, inp["t"], inp["ids"], inp["mask"])
-    loss = torch.nn.functional.mse_loss(pred, inp["noise"])
-    loss.backward()
-    return xt, pred.detach(), loss.detach(), {k: v.grad for k, v in sd.items() if v.requires_grad}
-
-
-def _oracle_autocast(cfg, sd, inp):
-    import ref_model
-    sd = {k: v.detach().clone().requires_grad_(v.is_floating_point() and "inv_freq" not in k) for k, v in sd.items()}
-    xt = ref_model.add_noise(inp["x0"], inp["noise"], inp["t"])
-    with torch.autocast("cuda", dtype=torch.bfloat16):
-        pred = ref_model.tts_forward(sd, cfg, xt, inp["t"], inp["ids"], inp["mask"])
-    torch.nn.functional.mse_loss(pred.float(), inp["noise"]).backward()
-    return {k: v.grad for k, v in sd.items() if v.requires_grad and v.grad is not None}
 
 
 # Sizes: the two toy configs at >= 272 (batch x frame) positions, `mid` = the real level-0/1 widths (320 / 640 channels, head dims
@@ -38,12 +19,9 @@ def _oracle_autocast(cfg, sd, inp):
 # 2e-2, which is why the toy cases are not run that small; the bar itself is not relaxed anywhere.
 @pytest.mark.parametrize("cfg_name,B,T", [("tiny", 8, 64), ("tiny3", 2, 136), ("tiny3", 8, 128), ("mid", 2, 64), ("1d_config", 2, 752)])
 def test_full_model_fwd_bwd(cuda, cfg_name, B, T):
-    from prompt_tts_b200.models import TTSSingleSpeaker
-    cfg = load_cfg(cfg_name)
-    torch.manual_seed(0)
-    model = TTSSingleSpeaker(cfg).to(cuda)
+    cfg, model = load_model(cfg_name, cuda, train=True)
     inp = synth_inputs(cfg, B, T, seed=1, device=cuda)
-    xt, ref_pred, ref_loss, ref_grads = _oracle(cfg, model.state_dict(), inp)
+    xt, ref_pred, ref_loss, ref_grads = to.oracle_train(cfg, model, inp)
 
     out = model(xt, inp["t"], inp["ids"], inp["mask"]).sample
     assert out.shape == ref_pred.shape and out.dtype == torch.float32
@@ -70,7 +48,7 @@ def test_full_model_fwd_bwd(cuda, cfg_name, B, T):
     gr = torch.cat([ref_grads[k].flatten() for _, k in worst])
     e_all = rel(gv, gr)
     # the reference's own bf16 path (torch.autocast) on the same inputs: the noise floor of bf16 compute at this depth
-    ac = _oracle_autocast(cfg, model.state_dict(), inp)
+    ac = to.oracle_train(cfg, model, inp, autocast=True)[3]
     gac = torch.cat([ac[k].flatten() for _, k in worst])
     e_ac = rel(gac, gr)
     print(f"\n[{cfg_name} B={B} T={T}] out {e_out:.2e} grad(all) {e_all:.2e} (reference under torch.autocast(bf16): {e_ac:.2e}) worst {worst[:4]}")
@@ -83,10 +61,7 @@ def test_full_model_fwd_bwd(cuda, cfg_name, B, T):
 
 
 def test_no_grad_inference_matches(cuda):
-    from prompt_tts_b200.models import TTSSingleSpeaker
-    cfg = load_cfg("tiny")
-    torch.manual_seed(0)
-    model = TTSSingleSpeaker(cfg).to(cuda).eval()
+    cfg, model = load_model("tiny", cuda)
     inp = synth_inputs(cfg, 2, 16, seed=3, device=cuda)
     with torch.no_grad():
         a = model(inp["x0"], inp["t"], inp["ids"], inp["mask"]).sample

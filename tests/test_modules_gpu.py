@@ -7,7 +7,8 @@ import torch
 import torch.nn.functional as F
 
 import ref_model
-from util import rel
+import training_oracle as to
+from util import load_model, rel, synth_inputs
 
 pytestmark = pytest.mark.gpu
 TOL = 2e-2
@@ -167,13 +168,9 @@ def test_mid_and_up_blocks_forward(cuda):
 def test_text_encoder_and_unet_forward(cuda):
     """TextEncoder.forward(input_ids, attention_mask) and Unet1DConditionModel.forward(sample, timestep, encoder_hidden_states, ...)
     called on their own (models.py:106-120, unet_1d_condition.py:553-739), timestep as tensor / 0-d tensor / int."""
-    from prompt_tts_b200.models import TTSSingleSpeaker
-    from util import load_cfg, synth_inputs
-    cfg = load_cfg("mid")
-    torch.manual_seed(0)
-    model = TTSSingleSpeaker(cfg).cuda()
+    cfg, model = load_model("mid", cuda, train=True)
     inp = synth_inputs(cfg, 2, 64, seed=5, device="cuda")
-    sd = {k: v.detach().clone().requires_grad_(v.is_floating_point() and "inv_freq" not in k) for k, v in model.state_dict().items()}
+    sd = to.oracle_params(model)
     enc = model.text_encoder(inp["ids"], inp["mask"])
     ref_enc = ref_model.text_encoder(sd, cfg, inp["ids"])
     assert rel(enc, ref_enc) < TOL

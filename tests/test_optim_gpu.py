@@ -4,23 +4,11 @@ lines train.py:41-47,116-120 -- applied to the same gradients, eagerly and repla
 import pytest
 import torch
 
-from util import load_cfg, rel, synth_inputs
+import training_oracle as to
+from util import load_model, rel
 
 pytestmark = pytest.mark.gpu
-KW = dict(lr=1e-3, betas=(0.95, 0.999), weight_decay=1e-2, eps=1e-8)     # lr large enough that a few steps move the weights measurably
-
-
-def _setup(cuda, B=2, T=16, seed=2, accumulation_steps=1, max_norm=0.05):
-    from prompt_tts_b200.models import TTSSingleSpeaker
-    from prompt_tts_b200.optim import FusedClipAdamW
-    from prompt_tts_b200.train import DenoiserTrainStep
-    cfg = load_cfg("tiny")
-    torch.manual_seed(0)
-    model = TTSSingleSpeaker(cfg).to(cuda)
-    inp = synth_inputs(cfg, B, T, seed=seed, device=cuda)
-    stepper = DenoiserTrainStep(model, accumulation_steps=accumulation_steps)
-    opt = FusedClipAdamW(stepper, max_norm=max_norm, **KW)       # clip threshold below the actual norm so clipping is active
-    return cfg, model, inp, stepper, opt
+KW = {k: v for k, v in to.OPT_KW.items() if k != "max_norm"}           # torch's AdamW takes no clip threshold
 
 
 class TorchRef:
@@ -44,7 +32,7 @@ class TorchRef:
 
 
 def test_fused_clip_adamw_matches_torch(cuda):
-    cfg, model, inp, stepper, opt = _setup(cuda)
+    cfg, model, inp, stepper, opt, _ = to.setup(cuda)
     ref = TorchRef(model, 0.05)
     for it in range(3):
         stepper(inp["x0"], inp["noise"], inp["t"], inp["ids"], inp["mask"])
@@ -71,7 +59,7 @@ def test_fused_clip_adamw_matches_torch(cuda):
 def test_fused_adamw_graph_replays(cuda):
     """One captured `step(); opt.step()` replayed: the step counter / bias corrections / clip factor / learning rate live in device
     memory, so every replay is the next optimiser step (round 1 baked step = 2 into the graph: updates ~0.46x the correct size)."""
-    cfg, model, inp, stepper, opt = _setup(cuda)
+    cfg, model, inp, stepper, opt, _ = to.setup(cuda)
     ref = TorchRef(model, 0.05)
 
     def full():
@@ -81,17 +69,8 @@ def test_fused_adamw_graph_replays(cuda):
     stepper(inp["x0"], inp["noise"], inp["t"], inp["ids"], inp["mask"])      # eager step 1 (defines the flat layout)
     ref.step(model)
     opt.step()
-    side = torch.cuda.Stream()                                                # warm-up on a side stream, as torch asks before capture
-    side.wait_stream(torch.cuda.current_stream())
-    with torch.cuda.stream(side):
-        stepper(inp["x0"], inp["noise"], inp["t"], inp["ids"], inp["mask"])
-        ref.step(model)
-        opt.step()
-    torch.cuda.current_stream().wait_stream(side)
-    torch.cuda.synchronize()
-    g = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(g):
-        full()
+    g = to.capture(full)
+    ref.step(model)                       # the warm-up step's gradients: opt.step() leaves param.grad as it is
     for it in range(5):
         if it == 3:                       # an LR scheduler writes the device-side learning rate between replays
             opt.set_lr(5e-4)
@@ -108,7 +87,7 @@ def test_fused_adamw_graph_replays(cuda):
 def test_gradient_accumulation_matches_one_big_batch(cuda):
     """Two micro-batches under accumulation_steps = 2 (`accelerator.accumulate`, train.py:27,80) == one step on the concatenated batch."""
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model, inp, stepper, opt = _setup(cuda, B=4, T=32)
+    cfg, model, inp, stepper, opt, _ = to.setup(cuda, B=4, T=32)
     big = DenoiserTrainStep(model)
     big(inp["x0"], inp["noise"], inp["t"], inp["ids"], inp["mask"])
     g_big = big.grad_sync.flat.clone()
@@ -126,13 +105,11 @@ def test_gradient_accumulation_matches_one_big_batch(cuda):
 
 
 def test_shadow_follows_load_state_dict_and_dtypes_are_converted(cuda):
-    from prompt_tts_b200.models import TTSSingleSpeaker
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model, inp, stepper, opt = _setup(cuda)
+    cfg, model, inp, stepper, opt, _ = to.setup(cuda)
     stepper(inp["x0"], inp["noise"], inp["t"], inp["ids"], inp["mask"])
     opt.step()
-    torch.manual_seed(7)
-    other = TTSSingleSpeaker(cfg).to(cuda)
+    _, other = load_model("tiny", cuda, train=True, seed=7)
     want = float(DenoiserTrainStep(other)(inp["x0"], inp["noise"], inp["t"], inp["ids"], inp["mask"]))
     model.load_state_dict(other.state_dict())            # in-place writes into the flat master buffer, from outside the optimiser
     got = float(stepper(inp["x0"], inp["noise"], inp["t"], inp["ids"], inp["mask"]))

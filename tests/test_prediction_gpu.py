@@ -9,8 +9,9 @@ import torch
 
 import prediction_oracle as po
 import sampling_oracle as so
+import training_oracle as to
 from prediction_oracle import DDIMScheduler, DDPMScheduler, DPMSolverMultistepScheduler
-from util import rel, synth_inputs
+from util import load_model, rel, synth_inputs
 
 pytestmark = pytest.mark.gpu
 TOL = 2e-2
@@ -257,7 +258,7 @@ def test_gaussian_target_kernel_loops_agree(cuda, kind, eta, n):
     """The samplers' own step code (`_step`, the fused kernels) driven by the exact predictor of x0 ~ N(0, 0.577^2), given as eps,
     x0 or v (computed in float64, rounded to fp32).  The three loops agree to 1e-5 (DESIGN section 5: an fp32 restatement of these
     steps keeps each parameterisation within 4e-7 of the float64 loop)."""
-    _, model = so.load_model("tiny", cuda)
+    _, model = load_model("tiny", cuda)
     B, C, T, s = 25, 8, 1000, 0.577
     g = torch.Generator(device="cuda").manual_seed(5)
     x_T = torch.randn(B, C, T, device=cuda, generator=g)
@@ -285,24 +286,16 @@ def test_gaussian_target_kernel_loops_agree(cuda, kind, eta, n):
 
 
 # ---------------------------------------------------------------------------------------------------------------- training
-def _oracle_train(cfg, model, inp, pt, gamma):
-    sd = {k: v.detach().clone().requires_grad_(v.is_floating_point() and "inv_freq" not in k) for k, v in model.state_dict().items()}
-    loss, _ = po.train_step_loss(sd, cfg, inp["x0"], inp["noise"], inp["t"], inp["ids"], inp["mask"], prediction_type=pt,
-                                 snr_gamma=gamma)
-    loss.backward()
-    return loss.detach(), {k: v.grad for k, v in sd.items() if v.requires_grad and v.grad is not None and v.grad.abs().max() > 0}
-
-
 # sizes: those of test_guidance_gpu.py's condition-dropout test (test_model_gpu.py gives the reason)
 @pytest.mark.parametrize("gamma", [None, 5.0])
 @pytest.mark.parametrize("pt", NON_EPS)
 @pytest.mark.parametrize("cfg_name,B,T", [("tiny", 8, 64), ("mid", 2, 64)])
 def test_train_step_prediction_type_matches_oracle(cuda, cfg_name, B, T, pt, gamma):
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = so.load_model(cfg_name, cuda, train=True)
+    cfg, model = load_model(cfg_name, cuda, train=True)
     inp = synth_inputs(cfg, B, T, seed=1, device=cuda)
     inp["t"][0] = 999
-    ref_loss, ref_grads = _oracle_train(cfg, model, inp, pt, gamma)
+    _, _, ref_loss, ref_grads = to.oracle_train(cfg, model, inp, prediction_type=pt, snr_gamma=gamma)
     loss = DenoiserTrainStep(model, prediction_type=pt, snr_gamma=gamma)(inp["x0"], inp["noise"], inp["t"], inp["ids"], inp["mask"])
     torch.cuda.synchronize()
     e_l, e_g = rel(loss, ref_loss), so.grad_err(model, ref_grads)
@@ -314,7 +307,7 @@ def test_train_step_graph_replays_fresh_timesteps(cuda):
     """the Min-SNR weight and the v target are formed on the device from t: replays of one captured step with two (t, noise) pairs
     equal eager steps with the same pairs"""
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = so.load_model("tiny", cuda, train=True)
+    cfg, model = load_model("tiny", cuda, train=True)
     B, T = 8, 64
     inp = synth_inputs(cfg, B, T, seed=4, device=cuda)
     stepper = DenoiserTrainStep(model, prediction_type="v_prediction", snr_gamma=5.0)
@@ -322,42 +315,15 @@ def test_train_step_graph_replays_fresh_timesteps(cuda):
     g = torch.Generator(device="cuda").manual_seed(8)
     pairs = [(inp["t"].clone(), inp["noise"].clone()),
              (torch.randint(0, 1000, (B,), device=cuda, generator=g), torch.randn(inp["noise"].shape, device=cuda, generator=g))]
-    loss = torch.zeros((), device=cuda)
-    named = list(model.named_parameters())
-
-    def step():
-        return stepper(inp["x0"], noise, t, inp["ids"], loss_out=loss)
-
-    eager = []
-    for tt, nn in pairs:
-        t.copy_(tt)
-        noise.copy_(nn)
-        step()
-        torch.cuda.synchronize()
-        eager.append((float(loss), torch.cat([p.grad.flatten() for _, p in named if p.grad is not None]).clone()))
-    side = torch.cuda.Stream()
-    side.wait_stream(torch.cuda.current_stream())
-    with torch.cuda.stream(side):
-        step()
-    torch.cuda.current_stream().wait_stream(side)
-    torch.cuda.synchronize()
-    graph = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(graph):
-        step()
-    for (tt, nn), (l_e, g_e) in zip(pairs, eager):
-        t.copy_(tt)
-        noise.copy_(nn)
-        graph.replay()
-        torch.cuda.synchronize()
-        gr = torch.cat([p.grad.flatten() for _, p in named if p.grad is not None])
-        assert abs(float(loss) - l_e) <= 1e-3 * abs(l_e) and rel(gr, g_e) < 1e-3
+    eager = to.check_replays_fresh_inputs(model, lambda loss: stepper(inp["x0"], noise, t, inp["ids"], loss_out=loss), [t, noise],
+                                          pairs)
     assert abs(eager[0][0] - eager[1][0]) > 1e-3 * abs(eager[0][0]), "the two pairs must give different losses"
 
 
 # ---------------------------------------------------------------------------------------------------------------- sampling loops
 @pytest.fixture(scope="module")
 def tiny(cuda):
-    return so.load_model("tiny", cuda)
+    return load_model("tiny", cuda)
 
 
 def _bound(model, cfg, kind, eta, n_infer, pt, w, inp, x_T, noises, want, prompt=None, pn=None):
@@ -444,7 +410,7 @@ def test_launch_counts(cuda, monkeypatch):
     """The default train step still launches add_noise + mse_fwd_bwd, a non-default one add_noise + diffusion_loss: the same count.
     Every sampler calls its `_pred` step entry point once per step whatever the type, and launches as many kernels for each type."""
     from prompt_tts_b200.train import DenoiserTrainStep
-    cfg, model = so.load_model("tiny", cuda, train=True)
+    cfg, model = load_model("tiny", cuda, train=True)
     B, T = 8, 64
     inp = synth_inputs(cfg, B, T, seed=9, device=cuda)
     counts = {}

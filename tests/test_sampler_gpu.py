@@ -4,7 +4,7 @@ import pytest
 import torch
 
 import sampling_oracle as so
-from util import rel, synth_inputs
+from util import load_model, rel, synth_inputs
 
 pytestmark = pytest.mark.gpu
 
@@ -28,7 +28,7 @@ def test_ddpm_step_matches_oracle(cuda, t):
 
 def test_sampler_matches_oracle_loop(cuda):
     from prompt_tts_b200.sample import DDPMSampler
-    cfg, model = so.load_model("tiny", cuda)
+    cfg, model = load_model("tiny", cuda)
     B, T, n_infer = 2, 16, 5
     inp = synth_inputs(cfg, B, T, seed=5, device=cuda)
     g = torch.Generator(device="cuda").manual_seed(9)
@@ -48,7 +48,7 @@ def test_sampler_matches_oracle_loop(cuda):
 
 def test_sampler_prompt_inpainting_and_codes(cuda):
     from prompt_tts_b200.sample import DDPMSampler
-    cfg, model = so.load_model("tiny", cuda)
+    cfg, model = load_model("tiny", cuda)
     B, T, P = 2, 16, 6
     inp = synth_inputs(cfg, B, T, seed=6, device=cuda)
     prompt = inp["x0"][..., :P].contiguous()
@@ -66,7 +66,7 @@ def test_sampler_prompt_tokens_extend_the_cross_attention_context(cuda):
     """Optional speech-prompt tokens appended to the text encoding (SURVEY 8 row N2 hook, default off): the run with tokens equals
     the oracle loop whose encoder_hidden_states is [text encoding | tokens], and differs from the run without them."""
     from prompt_tts_b200.sample import DDPMSampler
-    cfg, model = so.load_model("tiny", cuda)
+    cfg, model = load_model("tiny", cuda)
     B, T, n_infer, P = 2, 16, 3, 9
     inp = synth_inputs(cfg, B, T, seed=8, device=cuda)
     g = torch.Generator(device="cuda").manual_seed(4)

@@ -10,6 +10,15 @@ def load_cfg(name):
     return json.load(open(os.path.join(ROOT, "configs", name + ".json")))
 
 
+def load_model(cfg_name, dev, train=False, seed=0):
+    """the config and TTSSingleSpeaker(cfg) on dev with the weights torch.manual_seed(seed) draws, in eval mode unless train"""
+    from prompt_tts_b200.models import TTSSingleSpeaker
+    cfg = load_cfg(cfg_name)
+    torch.manual_seed(seed)
+    m = TTSSingleSpeaker(cfg).to(dev)
+    return cfg, (m if train else m.eval())
+
+
 def rel(a, b):
     a, b = a.detach().float(), b.detach().float()
     return ((a - b).norm() / (b.norm() + 1e-30)).item()

@@ -4,7 +4,7 @@ root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, root); sys.path.insert(0, os.path.join(root, "tests")); sys.path.insert(0, os.path.join(root, "oracle"))
 import torch
 from util import load_cfg, rel, synth_inputs
-import test_model_gpu as tm
+import training_oracle as to
 from prompt_tts_b200.models import TTSSingleSpeaker
 
 cfg_name, B, T = sys.argv[1], int(sys.argv[2]), int(sys.argv[3])
@@ -13,10 +13,10 @@ cfg = load_cfg(cfg_name)
 torch.manual_seed(0)
 model = TTSSingleSpeaker(cfg).to(cuda)
 inp = synth_inputs(cfg, B, T, seed=1, device=cuda)
-xt, ref_pred, ref_loss, ref_grads = tm._oracle(cfg, model.state_dict(), inp)
+xt, ref_pred, ref_loss, ref_grads = to.oracle_train(cfg, model, inp)
 out = model(xt, inp["t"], inp["ids"], inp["mask"]).sample
 torch.nn.functional.mse_loss(out.float(), inp["noise"].float()).backward()
-ac = tm._oracle_autocast(cfg, model.state_dict(), inp)
+ac = to.oracle_train(cfg, model, inp, autocast=True)[3]
 named = dict(model.named_parameters())
 rows = []
 tot_e = tot_r = tot_a = 0.0
